@@ -346,6 +346,31 @@ def microbench(hbm_gbs):
     return res
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, outs):
+    """What one step of the timed path hands its caller (engine.detect_graphed: boxes, masks,
+    scores, valid, and the RoI count per image) as float32 DIR/<name>.npy, so that two builds can
+    be compared output for output.  If the masks would take the total over 64 MB (batch 60 and
+    up), a fixed seeded sample of their rows is written instead, with the row numbers in
+    masks_rows.npy."""
+    import numpy as np
+    boxes, masks, scores, valid, o = outs
+    arrs = {name: t.float().cpu().numpy() for name, t in (
+        ("boxes", boxes), ("masks", masks), ("scores", scores), ("valid", valid), ("roi_counts", o["roi_counts"]))}
+    total = sum(a.nbytes for a in arrs.values())
+    if total > DUMP_LIMIT:
+        m = arrs["masks"]
+        flat = m.reshape(m.shape[0] * m.shape[1], -1)
+        n = (DUMP_LIMIT - (total - m.nbytes)) // (flat.shape[1] * 4 + 8)
+        rows = np.sort(np.random.default_rng(0).choice(flat.shape[0], n, replace=False))
+        arrs["masks"], arrs["masks_rows"] = flat[rows], rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -378,7 +403,11 @@ def main():
     ap.add_argument("--dump-igemm", default=None,
                     help="write the ordered list of tensor-core launches of one step "
                          "(shape, algorithmic FLOPs / bytes) as JSON, for scripts/ncu_tc_summary.py")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed (rank 0's images) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     _claim_stdout()
     # a run that is still going after 5 minutes leaves the Python stacks of all threads on stderr
     # (the default line takes ~20 s on a warm box; one run of the round stalled without a trace)
@@ -502,7 +531,7 @@ def main():
     ev[0].record()
     fork()
     for k in range(args.steps):
-        step_k(k)
+        last_outs, _ = step_k(k)
         if k + 1 < args.steps:
             ev[k + 1].record(streams[k % n_str] if n_str > 1 else None)
     join()
@@ -519,6 +548,9 @@ def main():
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
     total_ms = float(tms.item())
     value = world * B * args.steps / (total_ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        # before the passes below reuse the engines' output buffers
+        dump_outputs(args.dump_outputs, last_outs)
 
     # the collective alone (same buffers, main stream, nothing to overlap with)
     comm_ms = 0.0

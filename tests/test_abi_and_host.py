@@ -91,13 +91,13 @@ def test_prototxt_reader_and_graph_check(tmp_path):
     p.write_text(emit(mnc_graph.GRAPHS["cfm"](), ("data", "im_info")))
     with pytest.raises(ValueError):
         mnc_graph.identify_prototxt(str(p))           # CFM layers with the wrong inputs
-    base = "/root/reference/models/VGG16/"
-    if os.path.exists(base):  # build container only
-        assert len(mnc_graph.check_prototxt(base + "mnc_5stage/test.prototxt")) == 88
-        assert mnc_graph.identify_prototxt(base + "faster_rcnn_end2end/test.prototxt")[0] == "faster_rcnn"
-        assert mnc_graph.identify_prototxt(base + "cfm/test.prototxt")[0] == "cfm"
-        with pytest.raises(ValueError):
-            mnc_graph.identify_prototxt(base + "mnc_5stage/train.prototxt")
+    # the original project's own prototxts (models/VGG16/, copied unmodified)
+    base = os.path.join(ROOT, "tests", "golden", "models", "VGG16") + os.sep
+    assert len(mnc_graph.check_prototxt(base + "mnc_5stage/test.prototxt")) == 88
+    assert mnc_graph.identify_prototxt(base + "faster_rcnn_end2end/test.prototxt")[0] == "faster_rcnn"
+    assert mnc_graph.identify_prototxt(base + "cfm/test.prototxt")[0] == "cfm"
+    with pytest.raises(ValueError):
+        mnc_graph.identify_prototxt(base + "mnc_5stage/train.prototxt")
 
 
 def test_cfg_constants():
@@ -280,19 +280,19 @@ def test_hdf5_reader_on_reference_test_files_and_caffemodel_h5(tmp_path):
     B-tree spans several symbol-table nodes; (3) the engine weight dict from it."""
     from mnc_b200 import hdf5_min, weights as Wt, caffemodel as CM
     from tests.util import write_h5_tree
-    base = "/root/reference/caffe-mnc/src/caffe/test/test_data/"
-    if os.path.exists(base + "sample_data.h5"):   # build container only
-        data = np.arange(10 * 8 * 6 * 5).reshape(10, 8, 6, 5).astype(np.float32)
-        label = (1 + np.arange(10)[:, None]).astype(np.float32)
-        d = hdf5_min.read_hdf5(base + "sample_data.h5")
-        assert set(d) == {"/data", "/label", "/label2"}
-        assert np.array_equal(d["/data"], data) and np.array_equal(d["/label"], label)
-        assert np.array_equal(d["/label2"], label + 1)
-        g = hdf5_min.read_hdf5(base + "sample_data_2_gzip.h5")
-        assert np.array_equal(g["/data"], data + data.size) and g["/label"].dtype == np.uint8
-        assert np.array_equal(g["/label2"], (label + 1).astype(np.uint8))
-        s = hdf5_min.read_hdf5(base + "solver_data.h5")
-        assert s["/data"].shape == (8, 3, 10, 10) and s["/targets"].shape == (8, 1)
+    # caffe-mnc/src/caffe/test/test_data/*.h5, copied unmodified
+    base = os.path.join(ROOT, "tests", "golden", "caffe_test_data") + os.sep
+    data = np.arange(10 * 8 * 6 * 5).reshape(10, 8, 6, 5).astype(np.float32)
+    label = (1 + np.arange(10)[:, None]).astype(np.float32)
+    d = hdf5_min.read_hdf5(base + "sample_data.h5")
+    assert set(d) == {"/data", "/label", "/label2"}
+    assert np.array_equal(d["/data"], data) and np.array_equal(d["/label"], label)
+    assert np.array_equal(d["/label2"], label + 1)
+    g = hdf5_min.read_hdf5(base + "sample_data_2_gzip.h5")
+    assert np.array_equal(g["/data"], data + data.size) and g["/label"].dtype == np.uint8
+    assert np.array_equal(g["/label2"], (label + 1).astype(np.uint8))
+    s = hdf5_min.read_hdf5(base + "solver_data.h5")
+    assert s["/data"].shape == (8, 3, 10, 10) and s["/targets"].shape == (8, 1)
     w = Wt.make_weights(Wt.TINY_ARCH)
     tree = {"data": {}, "diff": {}}
     for name, (wt, b) in w.items():

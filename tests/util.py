@@ -55,6 +55,28 @@ def rel_err(a, b):
     return np.abs(a - b).max() / denom
 
 
+def digest(a):
+    """sha256 of an array's shape and values: for NaN-free arrays, equal digests <=> np.array_equal
+    (floats are hashed as float64 with -0.0 folded into +0.0, integers as int64)."""
+    import hashlib
+    a = np.asarray(a)
+    if a.dtype.kind == "f":
+        a = a.astype(np.float64) + 0.0
+    else:
+        a = a.astype(np.int64)
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(str(a.shape).encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def sample_idx(size, n=1024, seed=0):
+    """A fixed sample of n flat indices into an array of `size` elements (all of them if fewer)."""
+    if size <= n:
+        return np.arange(size)
+    return np.sort(np.random.default_rng(seed).choice(size, n, replace=False))
+
+
 # ---------------------------------------------------------------------------------------------
 # Test-only HDF5 assembler (superblock v0, old-style groups, contiguous float32 datasets): builds
 # files with NESTED groups and multi-node group B-trees byte by byte from the file-format
