@@ -27,6 +27,9 @@ class Detector:
         self._h_rec = torch.empty(ops.record_layout(B, ROIS_PER_IMAGE)[3], dtype=torch.float32).pin_memory()
         self._h_valid = torch.empty((B, n), dtype=torch.uint8).pin_memory()
         self._d_in = torch.empty((B, 3, height, width), dtype=torch.float32, device=self.device)
+        # the engine's per-tensor activation maxima come back with every record (512 B): each
+        # call checks them against the exponents the step ran with
+        self._h_amax = torch.empty_like(self.engine._amax_all, device="cpu").pin_memory()
         self.h2d_bytes = 0
         self.d2h_bytes = 0
 
@@ -63,26 +66,32 @@ class Detector:
         with torch.cuda.device(dev):
             self._d_in[:B].copy_(src, non_blocking=True)
             info = info_h.to(dev, non_blocking=True)
-            boxes, masks, scores, valid, _ = self._detect(
-                self._d_in[:B], info, hw_h.to(dev), scale_h.to(dev))
-            out = self._results_to_host(B, valid)
+            out = self._detect_to_host(B, self._d_in[:B], info, hw_h.to(dev), scale_h.to(dev))
         self.h2d_bytes = blob.numel() * 4 + info_h.numel() * 4 + scale_h.numel() * 4 + hw_h.numel() * 4
         return out
 
     def _detect(self, data, info, hw, sc):
-        # every 32nd call: did any activation outgrow the exponents frozen at calibration?
-        self._calls = getattr(self, "_calls", 0) + 1
-        if self._calls % 32 == 0:
-            self.engine.range_ok()
         if self.use_graph:
             return self.engine.detect_graphed(data, info, hw, sc)
         return self.engine.detect(data, info, hw, sc)
+
+    def _detect_to_host(self, B, data, info, hw, sc):
+        """One step, its results to host memory, then the range check on the activation maxima
+        that came back with them: a batch whose activations outgrew the frozen exponents
+        (MNCEngine.range_ok) is computed again with exponents measured on it."""
+        valid = self._detect(data, info, hw, sc)[3]
+        out = self._results_to_host(B, valid)
+        if not self.engine.range_ok(amax=self._h_amax):
+            valid = self._detect(data, info, hw, sc)[3]
+            out = self._results_to_host(B, valid)
+        return out
 
     def _results_to_host(self, B, valid):
         rec = self.engine.last_record
         n = rec.numel()
         self._h_rec[:n].copy_(rec, non_blocking=True)
         self._h_valid[:B].copy_(valid, non_blocking=True)
+        self._h_amax.copy_(self.engine._amax_all, non_blocking=True)
         torch.cuda.current_stream().synchronize()
         self.d2h_bytes = n * 4 + valid.numel()
         _, boxes, scores, masks = ops.record_views(self._h_rec[:n], B, ROIS_PER_IMAGE)
@@ -120,10 +129,8 @@ class Detector:
         with torch.cuda.device(dev):
             self._d_u8[:B].copy_(pinned_src, non_blocking=True)
             ops.prep_images(self._d_u8[:B], scale, out=self._d_in[:B])
-            boxes, masks, scores, valid, _ = self._detect(
-                self._d_in[:B], info.to(dev, non_blocking=True), hw.to(dev, non_blocking=True),
-                sc.to(dev, non_blocking=True))
-            out = self._results_to_host(B, valid)
+            out = self._detect_to_host(B, self._d_in[:B], info.to(dev, non_blocking=True),
+                                       hw.to(dev, non_blocking=True), sc.to(dev, non_blocking=True))
         self.h2d_bytes = images_u8.nbytes + (info.numel() + hw.numel() + sc.numel()) * 4
         return out + (scale,)
 
@@ -175,6 +182,7 @@ class Detector:
                       d_rec=torch.empty(n_rec, dtype=torch.float32, device=dev),
                       h_rec=torch.empty(n_rec, dtype=torch.float32).pin_memory(),
                       d_in=torch.empty_like(self._d_in),
+                      h_amax=torch.empty_like(self._h_amax).pin_memory(),
                       u8_free=None, out_done=None)
             self._slots[slot] = st
         if tuple(st["d_in"].shape) != tuple(self._d_in.shape):
@@ -206,33 +214,52 @@ class Detector:
             n = ops.record_layout(B, ROIS_PER_IMAGE)[3]
             args = (st["d_in"][:B], info.to(dev, non_blocking=True), hw.to(dev, non_blocking=True),
                     sc.to(dev, non_blocking=True))
-            self._calls = getattr(self, "_calls", 0) + 1
-            if self._calls % 32 in (0, 1) and self._calls > 1:
-                if not eng.range_ok():                              # exponents are shared: both re-measure
-                    for e in self._engines:
-                        if e is not None:
-                            e._calibrated = False
-                            e._graphs.clear() if hasattr(e, "_graphs") else None
-            if self.use_graph:
-                eng.detect_graphed(*args, rec=st["d_rec"])
-            else:
-                o = eng.forward(args[0], args[1])
-                eng.detect_tail(o, B, args[2], args[3], rec=st["d_rec"])
+            eng._amax_all.zero_()                                   # maxima of this step only
+            self._step(slot, args, B)
             ev_done = torch.cuda.Event()
             ev_done.record(main)
             with torch.cuda.stream(self._s_out):                    # record of this batch: D2H
                 self._s_out.wait_event(ev_done)
                 st["h_rec"][:n].copy_(st["d_rec"][:n], non_blocking=True)
+                st["h_amax"].copy_(eng._amax_all, non_blocking=True)
                 st["out_done"] = torch.cuda.Event()
                 st["out_done"].record(self._s_out)
         self.h2d_bytes = images_u8.nbytes + (info.numel() + hw.numel() + sc.numel()) * 4
         self.d2h_bytes = n * 4
-        return (slot, B, n, scale)
+        # the exponents this step ran with (a captured graph keeps those of its capture)
+        return (slot, B, n, scale, args, dict(eng.exp))
+
+    def _step(self, slot, args, B):
+        eng, st = self._engines[slot], self._slots[slot]
+        if self.use_graph:
+            eng.detect_graphed(*args, rec=st["d_rec"])
+        else:
+            o = eng.forward(args[0], args[1])
+            eng.detect_tail(o, B, args[2], args[3], rec=st["d_rec"])
 
     def _collect(self, handle):
-        slot, B, n, scale = handle
-        st = self._slots[slot]
+        slot, B, n, scale, args, exp_used = handle
+        st, eng = self._slots[slot], self._engines[slot]
         st["out_done"].synchronize()
+        # exponents re-measured since this batch was issued (on the other slot's batch): recompute
+        # it with the current ones; activations that outgrew the exponents: re-measure and recompute
+        ok = exp_used == eng.exp and eng.range_ok(reset=False, amax=st["h_amax"], exp=exp_used)
+        for _ in range(2):
+            if ok:
+                break
+            dev = self.device
+            # the other slot's step may still be replaying a graph that is about to be dropped
+            torch.cuda.synchronize(dev)
+            if not eng._calibrated:            # the exponents (shared by both slots) will change
+                for e in self._engines:
+                    if e is not None and hasattr(e, "_graphs"):
+                        e._graphs.clear()
+            with torch.cuda.device(dev), torch.cuda.stream(self._s_comp[slot]):
+                eng._amax_all.zero_()
+                self._step(slot, args, B)
+                st["h_rec"][:n].copy_(st["d_rec"][:n])
+            torch.cuda.synchronize(dev)
+            ok = eng.range_ok()
         counts, boxes, scores, masks = ops.record_views(st["h_rec"][:n], B, ROIS_PER_IMAGE)
         # valid flags from the counts (2 x RoIs per image: stage-1 rows, then stage-2 rows)
         per_stage = (counts.numpy() / 2).astype(np.int64)

@@ -33,6 +33,19 @@ def _ceil_half(x):
 
 HALO_MAX_COUT = 128    # 3x3 convs with Cout <= 128 run the halo kernel
 
+# Largest max |value| * 2^exp a tri-plane tensor may reach before its exponent counts as stale.
+# Calibration puts the maximum in (2^11, 2^12].  fp16 itself saturates only at 65504, but the e4m3
+# planes give out much earlier: the residual plane (x 2^6) clamps at 448 once the fp16 rounding
+# step exceeds 16 (values above 2^15), the copy plane (x 2^-5) above 14336, and the layer then
+# degrades toward plain fp16 (2e-4 per layer).  Up to 2^14 every layer kind stays within 1e-4 of
+# fp64 (tests/test_tri_headroom.py, tests/test_gpu_tri_path.py::test_headroom_contract).
+RANGE_MAX = 2.0 ** 14
+
+
+def in_range(amax, exp):
+    """Is a tensor whose max |value| is `amax` still carried accurately with exponent `exp`?"""
+    return amax * 2.0 ** exp <= RANGE_MAX
+
 
 def pick_split_k(tiles_m, tiles_n, k_steps, sms, cluster=2, max_split=32, out_elems=0):
     """Split-K only when the launch cannot fill the GPU (e.g. fc6_maskest: 19 row tiles,
@@ -126,6 +139,7 @@ class MNCEngine:
         # key): written by the producing kernels on every call, read by range_ok()
         self._amax_all = torch.zeros(128, dtype=torch.int32, device=dev)
         self._amax_slot = {}
+        self.range_violations = 0      # how often range_ok() found a stale exponent
         # the box branch (fc6 on the 7x7 features: tensor-bound) is issued on a side stream so that
         # the mask branch's small / HBM-bound kernels (mask_pred, sigmoid + resize, MaskPooling) run
         # under it instead of in front of it; in a captured graph the fork becomes parallel branches
@@ -178,8 +192,8 @@ class MNCEngine:
     def _scaled(self, exp_key, fn):
         """Run fn(out_exp, amax) -- the launch(es) that write the tri-plane tensor `exp_key`.  Normal
         operation: the frozen exponent.  Calibration (first forward): launch, read the measured
-        max |value|, choose the exponent that puts it at 2^12 (fp16 has 16x headroom above, the
-        e4m3 planes saturate gracefully), relaunch if it changed."""
+        max |value|, choose the exponent that puts it at 2^12 (4x headroom to RANGE_MAX, where the
+        e4m3 correction planes start to saturate), relaunch if it changed."""
         if not self._calibrating:
             slot = self._amax_slot.setdefault(exp_key, len(self._amax_slot))
             fn(self.exp[exp_key], self._amax_all[slot:slot + 1] if slot < 128 else None)
@@ -194,25 +208,45 @@ class MNCEngine:
         if e != e0:
             fn(e, None)
 
-    def range_ok(self, reset=True):
-        """Were the frozen exponents still adequate for everything computed since the last check?
-        One small D2H read.  A tensor whose maximum left the fp16 range of its exponent (value *
-        2^exp > 6e4: the main operand saturates) makes this return False and un-calibrates the
-        engine: the next forward measures the exponents again (and graphs are re-captured)."""
+    def range_ok(self, reset=True, amax=None, exp=None):
+        """Were the exponents still adequate for everything computed since the last check?  A
+        tensor whose maximum left the accurate range of its exponent (`in_range`) makes this return
+        False and un-calibrates the engine: the next forward measures the exponents again (and
+        graphs are re-captured).  amax: a host copy of `_amax_all` taken after the step (default:
+        one small D2H read now); exp: the exponents the step ran with (default: the current ones)."""
         if not self.tri or not self._amax_slot:
             return True
-        amax = self._amax_all.cpu().view(torch.float32)
+        amax = (self._amax_all.cpu() if amax is None else amax).view(torch.float32)
+        exp = self.exp if exp is None else exp
         bad = [k for k, i in self._amax_slot.items()
-               if i < 128 and float(amax[i]) * 2.0 ** self.exp.get(k, 0) > 6.0e4]
+               if i < 128 and not in_range(float(amax[i]), exp.get(k, 0))]
         if reset:
             self._amax_all.zero_()
         if bad:
+            self.range_violations += 1
             self._calibrated = False
             if hasattr(self, "_graphs"):
                 self._graphs.clear()
             self.last_range_violation = bad
             return False
         return True
+
+    def run_checked(self, step, *args, **kwargs):
+        """step(*args, **kwargs) -- this engine's forward, detect or detect_graphed -- followed by
+        the range check (one host sync); a batch whose activations outgrew the frozen exponents is
+        computed again with exponents measured on it.  Returns what the last step returned."""
+        out = step(*args, **kwargs)
+        if not self.range_ok():
+            out = step(*args, **kwargs)
+        return out
+
+    def forward_checked(self, data, im_info, keep_intermediate=False):
+        """`forward` with the per-call range check of `run_checked`."""
+        return self.run_checked(self.forward, data, im_info, keep_intermediate)
+
+    def detect_checked(self, data, im_info, im_hw, im_scale):
+        """`detect` with the per-call range check of `run_checked`."""
+        return self.run_checked(self.detect, data, im_info, im_hw, im_scale)
 
     def _f32_buf(self, key, *shape):
         t = self._buf.get(key)

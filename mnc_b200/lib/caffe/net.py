@@ -98,11 +98,12 @@ class Net(object):
             if self.kind == "faster_rcnn":
                 if self.blobs["data"].data.shape[0] != 1:
                     raise AssertionError("Only single item batches are supported")
-                o = self._engine.forward(t("data"), t("im_info"), keep_intermediate=True)
+                o = self._engine.forward_checked(t("data"), t("im_info"), keep_intermediate=True)
                 n = int(o["roi_counts"][0].item())
                 host = {"rois": o["rois"][:n], "cls_prob": o["cls_prob"][:n], "bbox_pred": o["bbox_pred"][:n]}
             else:
-                o = self._engine.forward(t("data"), t("rois"), t("masks"), keep_intermediate=True)
+                o = self._engine.run_checked(self._engine.forward, t("data"), t("rois"), t("masks"),
+                                             keep_intermediate=True)
                 R = self.blobs["rois"].data.shape[0]
                 host = {"mask_prob": o["mask_prob"].view(R, -1), "cls_prob": o["cls_prob"],
                         "seg_cls_prob": o["seg_cls_prob"], "bbox_pred": o["bbox_pred"]}
@@ -135,7 +136,7 @@ class Net(object):
         with torch.cuda.device(dev):
             d = torch.from_numpy(np.ascontiguousarray(data, dtype=np.float32)).to(dev)
             info = torch.from_numpy(np.ascontiguousarray(im_info, dtype=np.float32)).to(dev)
-            o = self._engine.forward(d, info, keep_intermediate=True)
+            o = self._engine.forward_checked(d, info, keep_intermediate=True)
             n = int(o["roi_counts"][0].item())
             conv5 = o["_conv5_3"]
             B, H5, W5, C5 = tuple(conv5.shape)[-4:]   # split bf16 [2, B, H, W, C] or dense.Tri

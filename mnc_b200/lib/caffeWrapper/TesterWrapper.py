@@ -108,7 +108,7 @@ class TesterWrapper(object):
             info = torch.tensor([[out_h, out_w, scale]] * B, dtype=torch.float32, device=dev)
             hw = torch.tensor([[H, W]] * B, dtype=torch.float32, device=dev)
             sc = torch.full((B,), scale, dtype=torch.float32, device=dev)
-            scores, pred, valid, _ = self.engine.detect(data, info, hw, sc)
+            scores, pred, valid, _ = self.engine.detect_checked(data, info, hw, sc)
             return scores.cpu().numpy(), pred.cpu().numpy(), valid.cpu().numpy().astype(bool)
 
     def _detection_forward(self, im):
@@ -179,8 +179,9 @@ class TesterWrapper(object):
                     rois = b_scale[s:s + max_rois].astype(np.float32, copy=False)
                     m_in = (m_scale[s:s + max_rois].reshape(-1, 1, S, S).astype(np.float32)
                             >= cfg.BINARIZE_THRESH).astype(np.float32)
-                    o = self.engine.forward(d_data, torch.from_numpy(np.ascontiguousarray(rois)).to(dev),
-                                            torch.from_numpy(m_in).to(dev))
+                    o = self.engine.run_checked(
+                        self.engine.forward, d_data, torch.from_numpy(np.ascontiguousarray(rois)).to(dev),
+                        torch.from_numpy(m_in).to(dev))
                     res_masks = np.vstack((res_masks, o["mask_prob"].cpu().numpy().reshape(
                         -1, 1, cfg.MASK_SIZE, cfg.MASK_SIZE)))
                     res_scores = np.vstack((res_scores, o["seg_cls_prob"].cpu().numpy()))
@@ -261,7 +262,7 @@ class TesterWrapper(object):
             info = torch.tensor([[out_h, out_w, scale]] * B, dtype=torch.float32, device=dev)
             hw = torch.tensor([[H, W]] * B, dtype=torch.float32, device=dev)
             sc = torch.full((B,), scale, dtype=torch.float32, device=dev)
-            boxes, masks, scores, valid, _ = det.engine.detect(det._d_in[:B], info, hw, sc)
+            boxes, masks, scores, valid, _ = det.engine.detect_checked(det._d_in[:B], info, hw, sc)
             vote = det.mask_voting(boxes, masks, scores, valid, [[H, W]] * B,
                                    max_per_image=self.max_per_image)
             return unpack_voting(vote, self.num_classes)

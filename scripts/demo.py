@@ -64,7 +64,7 @@ def main():
             info = torch.tensor([[out_h, out_w, scale]] * B, dtype=torch.float32, device=dev)
             hw = torch.tensor([[H, W]] * B, dtype=torch.float32, device=dev)
             sc = torch.full((B,), scale, dtype=torch.float32, device=dev)
-            boxes, masks, scores, valid, _ = det.engine.detect(det._d_in[:B], info, hw, sc)
+            boxes, masks, scores, valid, _ = det.engine.detect_checked(det._d_in[:B], info, hw, sc)
             vote = det.mask_voting(boxes, masks, scores, valid, [[H, W]] * B, max_per_image=100)
             vb, vm, vc, cnt = ops.select_for_display(vote, vis_thresh=args.vis_thresh)
             inst, cls, bgr = ops.paste_instances(vb, vm, vc, cnt, H, W, want_bgr=True)
