@@ -74,6 +74,57 @@ int mnc_igemm_tc2(int in_fmt, const void* a0, const void* a1, const void* a2, in
                   int bn, int max_ctas, float acc_scale, float out_scale, unsigned int* amax,
                   void* stream);
 
+/* Mixed-size batches.  Image b of the batch fills the top-left corner of the zero-padded blob;
+ * img_hw is a DEVICE int32 [batch][2] array of the images' sizes at input resolution (blob rows
+ * and columns of image b before any pooling), and `level` the number of 2x2 ceil-mode pools
+ * between the input and this launch (0 = conv1_x ... 4 = conv5_x / RPN), so that image b covers
+ * ((h + 2^level - 1) >> level, (w + 2^level - 1) >> level) of the launch's map.  img_hw lives in
+ * device memory, so these entry points check only `level` (MNC_ERR_ARG outside 0..16) and do NOT
+ * validate the sizes: the CALLER owns that check and must reject, on the host before uploading,
+ * any size < 1 or larger than the blob (the Python layer does so in engine.check_extents).  Invalid
+ * sizes give wrong results but never an out-of-map access: the kernels clamp every extent to the
+ * map (the RoI warps to [1, map]).  img_hw == NULL is the whole-blob launch of the entry point
+ * without the suffix.
+ *
+ * mnc_igemm_tc3: mnc_igemm_tc2 whose outputs outside their image are exact zeros (out_mode 0 / 4);
+ * with the fused pool (2 / 5) pixels outside the image take no part in a window and pooled pixels
+ * outside the image's level + 1 extent are zeros.  Running maxima (amax) count pixels inside. */
+int mnc_igemm_tc3(int in_fmt, const void* a0, const void* a1, const void* a2, int batch, int H,
+                  int W, int Cin, const void* w0, const void* w1, const void* w2, int Cout, int taps,
+                  const float* bias, int relu, int out_mode, void* out0, void* out1, void* out2,
+                  long long out_pix_stride, int out_ch_offset, int split_k, long long split_stride,
+                  int bn, int max_ctas, float acc_scale, float out_scale, unsigned int* amax,
+                  const int* img_hw, int level, void* stream);
+/* Split-K reductions of a conv launch over a [batch][H][W] map (rows = batch*H*W) with the rows
+ * outside their image written as zeros. */
+int mnc_splitk_reduce2(const float* partial, int splits, long long split_stride, long long rows,
+                       int cols, const float* bias, int relu, int out_mode, void* out0, void* out1,
+                       long long out_row_stride, int out_ch_offset, const int* img_hw, int level,
+                       int H, int W, void* stream);
+int mnc_splitk_reduce_tri2(const float* partial, int splits, long long split_stride, long long rows,
+                           int cols, const float* bias, int relu, float scale, void* h, void* l,
+                           void* c, long long out_row_stride, int out_ch_offset, unsigned int* amax,
+                           const int* img_hw, int level, int H, int W, void* stream);
+/* conv1_1 (level 0) of a mixed-size batch. */
+int mnc_conv1_1_tc3(const float* data_nchw, int batch, int H, int W, const void* w_stacked,
+                    const float* bias, int out_mode, void* out0, void* out1, void* out2,
+                    float out_scale, unsigned int* amax, const int* img_hw, void* stream);
+/* Proposal decode: anchors outside their image's extent are marked invalid. */
+int mnc_rpn_decode2(const float* cls, long long cls_img_stride, long long cls_ch_stride,
+                    long long cls_pix_stride, const float* bbox, long long bb_img_stride,
+                    long long bb_ch_stride, long long bb_pix_stride, const float* im_info, int batch,
+                    int H, int W, int feat_stride, float min_size, int apply_softmax,
+                    float* proposals, float* scores, unsigned char* valid, const int* img_hw,
+                    int level, void* stream);
+/* RoI warps: samples are bounded and clamped by the extent of the RoI's image (roi[0]); the map's
+ * row stride stays W.  Not combined with the A/B kernel forms (set_walk / set_rows): MNC_ERR_ARG. */
+int mnc_roi_warp_split2(const float* feat_nhwc, int C, int H, int W, const float* rois, int R,
+                        int sub, float spatial_scale, void* o14_hi, void* o14_lo, void* o7_hi,
+                        void* o7_lo, const int* img_hw, int level, void* stream);
+int mnc_roi_warp_tri2(const float* feat_nhwc, int C, int H, int W, const float* rois, int R, int sub,
+                      float spatial_scale, float scale, void* o14_h, void* o14_l, void* o14_c,
+                      void* o7_h, void* o7_l, void* o7_c, const int* img_hw, int level, void* stream);
+
 /* Tri-plane helpers.  fp32 -> (fp16 h, e4m3 l, e4m3 c) with scale 2^e and back (h + l / 2^6) *
  * inv_scale; n % 4 == 0. */
 int mnc_f32_to_tri(const float* in, long long n, float scale, void* h, void* l, void* c,
@@ -336,6 +387,15 @@ int mnc_mv_set_shape(int stride, int chunks_coarse, int chunks_border);
 int mnc_prep_images(const unsigned char* img_bgr_hwc, int batch, int H, int W,
                     const double* pixel_means3, double scale, int out_h, int out_w,
                     float* out_nchw, void* stream);
+/* Images of different sizes in one launch (im_list_to_blob, lib/utils/blob.py:17-31): image b,
+ * uint8 BGR HWC of src_hw[b] = (h, w) at byte offset offsets[b] of the DEVICE buffer `packed`, is
+ * prepared as mnc_prep_images does with scale scales[b] into the top-left dst_hw[b] (= its rounded
+ * scaled size) of the [batch][3][out_h][out_w] blob; every other blob element is written as 0.
+ * offsets, src_hw, scales, dst_hw: HOST arrays; batch <= 64. */
+int mnc_prep_images_ragged(const unsigned char* packed, int batch, const long long* offsets,
+                           const int* src_hw, const double* scales, const int* dst_hw,
+                           const double* pixel_means3, int out_h, int out_w, float* out_nchw,
+                           void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Result rendering (SURVEY.md section 8f, "next" row 3): _convert_pred_to_image

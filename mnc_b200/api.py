@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import ops
-from .engine import MNCEngine, ROIS_PER_IMAGE, MASK_SIZE, NUM_CLASSES
+from .engine import MNCEngine, ROIS_PER_IMAGE, MASK_SIZE, NUM_CLASSES, check_extents
 
 
 class Detector:
@@ -70,19 +70,19 @@ class Detector:
         self.h2d_bytes = blob.numel() * 4 + info_h.numel() * 4 + scale_h.numel() * 4 + hw_h.numel() * 4
         return out
 
-    def _detect(self, data, info, hw, sc):
+    def _detect(self, data, info, hw, sc, ext=None):
         if self.use_graph:
-            return self.engine.detect_graphed(data, info, hw, sc)
-        return self.engine.detect(data, info, hw, sc)
+            return self.engine.detect_graphed(data, info, hw, sc, extents=ext)
+        return self.engine.detect(data, info, hw, sc, extents=ext)
 
-    def _detect_to_host(self, B, data, info, hw, sc):
+    def _detect_to_host(self, B, data, info, hw, sc, ext=None):
         """One step, its results to host memory, then the range check on the activation maxima
         that came back with them: a batch whose activations outgrew the frozen exponents
         (MNCEngine.range_ok) is computed again with exponents measured on it."""
-        valid = self._detect(data, info, hw, sc)[3]
+        valid = self._detect(data, info, hw, sc, ext)[3]
         out = self._results_to_host(B, valid)
         if not self.engine.range_ok(amax=self._h_amax):
-            valid = self._detect(data, info, hw, sc)[3]
+            valid = self._detect(data, info, hw, sc, ext)[3]
             out = self._results_to_host(B, valid)
         return out
 
@@ -134,9 +134,72 @@ class Detector:
         self.h2d_bytes = images_u8.nbytes + (info.numel() + hw.numel() + sc.numel()) * 4
         return out + (scale,)
 
+    def _mixed_batch(self, images):
+        """Host side of a mixed-size batch: validation, per-image scales and blob sizes, the
+        packed frames in pinned staging `buf` (grown on demand).  -> dict of host values."""
+        images = [np.ascontiguousarray(im.numpy() if isinstance(im, torch.Tensor) else im)
+                  for im in images]
+        if not 1 <= len(images) <= self.max_batch:
+            raise ValueError("%d images in one batch, at most %d" % (len(images), self.max_batch))
+        for im in images:
+            if im.dtype != np.uint8 or im.ndim != 3 or im.shape[2] != 3 or min(im.shape[:2]) < 1:
+                raise ValueError("images must be uint8 BGR (H, W, 3) arrays, got %s %s" % (im.dtype, im.shape))
+        scales = np.array([ops.im_scale_for(im.shape) for im in images], dtype=np.float64)
+        src_hw = np.array([im.shape[:2] for im in images], dtype=np.int32)
+        dst_hw = np.array([ops.blob_size_for(im.shape, s) for im, s in zip(images, scales)], dtype=np.int32)
+        Hb, Wb = int(dst_hw[:, 0].max()), int(dst_hw[:, 1].max())
+        ext = check_extents(dst_hw, Hb, Wb, self.max_batch)
+        sizes = [im.nbytes for im in images]
+        offsets = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
+        return dict(images=images, scales=scales, src_hw=src_hw, dst_hw=dst_hw, H=Hb, W=Wb, ext=ext,
+                    offsets=offsets, nbytes=int(sum(sizes)), B=len(images))
+
+    @staticmethod
+    def _pack(mb, h_buf, dev, d_buf):
+        """Grow-on-demand pinned / device byte buffers holding the packed frames of `mb`."""
+        if h_buf is None or h_buf.numel() < mb["nbytes"]:
+            h_buf = torch.empty(mb["nbytes"], dtype=torch.uint8).pin_memory()
+            d_buf = torch.empty(mb["nbytes"], dtype=torch.uint8, device=dev)
+        for im, off in zip(mb["images"], mb["offsets"]):
+            h_buf[off:off + im.nbytes].copy_(torch.from_numpy(im.reshape(-1)))
+        return h_buf, d_buf
+
+    def _mixed_inputs(self, mb):
+        """im_info [blob h, blob w, scale], original sizes and scales of a mixed batch (host)."""
+        info = torch.tensor([[h, w, s] for (h, w), s in zip(mb["dst_hw"], mb["scales"])], dtype=torch.float32)
+        hw = torch.from_numpy(mb["src_hw"].astype(np.float32))
+        sc = torch.from_numpy(mb["scales"].astype(np.float32))
+        return info, hw, sc
+
+    def im_detect_mixed(self, images):
+        """`im_detect` on a batch of images of DIFFERENT sizes in one step: images is a list of
+        at most max_batch uint8 BGR (H_i, W_i, 3) host arrays.  Each image is scaled by its own
+        600/1000 rule and placed in the top-left corner of one zero-padded blob (as the
+        reference's `im_list_to_blob` pads), and every layer treats the pixels outside an image as
+        outside it, so each image gets the results it would get alone.  Returns boxes (in each
+        image's original coordinates), masks, scores, valid -- host arrays as `im_detect_images`
+        returns them -- and the scales (B,)."""
+        mb = self._mixed_batch(images)
+        B, dev = mb["B"], self.device
+        self._fit_input(mb["H"], mb["W"])
+        self._h_pack, self._d_pack = self._pack(mb, getattr(self, "_h_pack", None), dev,
+                                                getattr(self, "_d_pack", None))
+        info, hw, sc = self._mixed_inputs(mb)
+        with torch.cuda.device(dev):
+            self._d_pack[:mb["nbytes"]].copy_(self._h_pack[:mb["nbytes"]], non_blocking=True)
+            ops.prep_images_ragged(self._d_pack, mb["offsets"], mb["src_hw"], mb["scales"], mb["H"],
+                                   mb["W"], out=self._d_in[:B])
+            out = self._detect_to_host(B, self._d_in[:B], info.to(dev, non_blocking=True),
+                                       hw.to(dev, non_blocking=True), sc.to(dev, non_blocking=True),
+                                       mb["ext"].to(dev, non_blocking=True))
+        self.h2d_bytes = mb["nbytes"] + (info.numel() + hw.numel() + sc.numel() + mb["ext"].numel()) * 4
+        return out + (mb["scales"].copy(),)
+
     def im_detect_stream(self, batches):
         """Pipelined `im_detect_images`: an iterable of uint8 BGR (B,H,W,3) host batches (all of
-        one size) -> a generator of (boxes, masks, scores, valid, scale) per batch, in order.
+        one size) -> a generator of (boxes, masks, scores, valid, scale) per batch, in order.  A
+        batch may also be a LIST of differently sized (H_i, W_i, 3) images (`im_detect_mixed`);
+        its result then carries the scales (B,) in place of the scalar.
         Two batches are in flight: while batch k computes, the frames of batch k+1 cross PCIe on a
         copy stream and the record of batch k-1 comes back on another, so the host<->device copies
         (14.4 MB in, 9 MB out per batch of 8) leave the critical path; and the two batches compute
@@ -161,6 +224,8 @@ class Detector:
             yield self._collect(pending)
 
     def _submit(self, slot, images_u8):
+        if isinstance(images_u8, (list, tuple)):
+            return self._submit_mixed(slot, images_u8)
         dev = self.device
         pinned_src = None
         if isinstance(images_u8, torch.Tensor):
@@ -174,12 +239,27 @@ class Detector:
         scale = ops.im_scale_for((H, W))
         out_h, out_w = int(np.rint(H * scale)), int(np.rint(W * scale))
         self._fit_input(out_h, out_w)
+        st, eng = self._slot(slot)
+        if st.get("h_u8") is None or tuple(st["h_u8"].shape[1:]) != (H, W, 3):
+            st["h_u8"] = torch.empty((self.max_batch, H, W, 3), dtype=torch.uint8).pin_memory()
+            st["d_u8"] = torch.empty((self.max_batch, H, W, 3), dtype=torch.uint8, device=dev)
+        if pinned_src is None:
+            st["h_u8"][:B].copy_(torch.from_numpy(images_u8))      # pageable -> pinned staging (host)
+            pinned_src = st["h_u8"][:B]
+        info = torch.tensor([[out_h, out_w, scale]] * B, dtype=torch.float32)
+        hw = torch.tensor([[H, W]] * B, dtype=torch.float32)
+        sc = torch.full((B,), scale, dtype=torch.float32)
+        prep = lambda: ops.prep_images(st["d_u8"][:B], scale, out=st["d_in"][:B])
+        return self._issue(slot, st, eng, B, lambda: st["d_u8"][:B].copy_(pinned_src, non_blocking=True),
+                           prep, info, hw, sc, None, scale, images_u8.nbytes)
+
+    def _slot(self, slot):
+        """Slot `slot`'s staging buffers (input blob sized like _d_in) and engine."""
+        dev = self.device
         st = self._slots[slot]
-        if st is None or tuple(st["h_u8"].shape[1:]) != (H, W, 3):
+        if st is None:
             n_rec = ops.record_layout(self.max_batch, ROIS_PER_IMAGE)[3]
-            st = dict(h_u8=torch.empty((self.max_batch, H, W, 3), dtype=torch.uint8).pin_memory(),
-                      d_u8=torch.empty((self.max_batch, H, W, 3), dtype=torch.uint8, device=dev),
-                      d_rec=torch.empty(n_rec, dtype=torch.float32, device=dev),
+            st = dict(d_rec=torch.empty(n_rec, dtype=torch.float32, device=dev),
                       h_rec=torch.empty(n_rec, dtype=torch.float32).pin_memory(),
                       d_in=torch.empty_like(self._d_in),
                       h_amax=torch.empty_like(self._h_amax).pin_memory(),
@@ -191,29 +271,44 @@ class Detector:
         if eng is None:          # slot 1's engine: made once slot 0's first call has calibrated
             torch.cuda.synchronize(dev)
             eng = self._engines[slot] = self.engine.clone_state()
-        if pinned_src is None:
-            st["h_u8"][:B].copy_(torch.from_numpy(images_u8))      # pageable -> pinned staging (host)
-            pinned_src = st["h_u8"][:B]
-        info = torch.tensor([[out_h, out_w, scale]] * B, dtype=torch.float32)
-        hw = torch.tensor([[H, W]] * B, dtype=torch.float32)
-        sc = torch.full((B,), scale, dtype=torch.float32)
+        return st, eng
+
+    def _submit_mixed(self, slot, images):
+        mb = self._mixed_batch(images)
+        B = mb["B"]
+        self._fit_input(mb["H"], mb["W"])
+        st, eng = self._slot(slot)
+        if st["u8_free"] is not None:
+            st["u8_free"].synchronize()          # the pinned pack buffer may still be crossing
+        st["h_pack"], st["d_pack"] = self._pack(mb, st.get("h_pack"), self.device, st.get("d_pack"))
+        info, hw, sc = self._mixed_inputs(mb)
+        nb = mb["nbytes"]
+        h2d = lambda: st["d_pack"][:nb].copy_(st["h_pack"][:nb], non_blocking=True)
+        prep = lambda: ops.prep_images_ragged(st["d_pack"], mb["offsets"], mb["src_hw"], mb["scales"],
+                                              mb["H"], mb["W"], out=st["d_in"][:B])
+        return self._issue(slot, st, eng, B, h2d, prep, info, hw, sc, mb["ext"], mb["scales"].copy(), nb)
+
+    def _issue(self, slot, st, eng, B, h2d, prep, info, hw, sc, ext, scale, in_bytes):
+        """Queue one batch on slot `slot`: frames H2D on the copy stream (h2d), preparation (prep)
+        and the step on the slot's compute stream, the record D2H on the other copy stream."""
+        dev = self.device
         with torch.cuda.device(dev), torch.cuda.stream(self._s_comp[slot]):
             main = torch.cuda.current_stream()                      # this slot's compute stream
             with torch.cuda.stream(self._s_in):                     # frames of this batch: H2D
                 if st["u8_free"] is not None:
                     self._s_in.wait_event(st["u8_free"])
-                st["d_u8"][:B].copy_(pinned_src, non_blocking=True)
+                h2d()
                 ev_in = torch.cuda.Event()
                 ev_in.record(self._s_in)
             main.wait_event(ev_in)
-            ops.prep_images(st["d_u8"][:B], scale, out=st["d_in"][:B])
+            prep()
             st["u8_free"] = torch.cuda.Event()
             st["u8_free"].record(main)
             if st["out_done"] is not None:
                 main.wait_event(st["out_done"])                     # this slot's record was read
             n = ops.record_layout(B, ROIS_PER_IMAGE)[3]
             args = (st["d_in"][:B], info.to(dev, non_blocking=True), hw.to(dev, non_blocking=True),
-                    sc.to(dev, non_blocking=True))
+                    sc.to(dev, non_blocking=True), None if ext is None else ext.to(dev, non_blocking=True))
             eng._amax_all.zero_()                                   # maxima of this step only
             self._step(slot, args, B)
             ev_done = torch.cuda.Event()
@@ -224,7 +319,7 @@ class Detector:
                 st["h_amax"].copy_(eng._amax_all, non_blocking=True)
                 st["out_done"] = torch.cuda.Event()
                 st["out_done"].record(self._s_out)
-        self.h2d_bytes = images_u8.nbytes + (info.numel() + hw.numel() + sc.numel()) * 4
+        self.h2d_bytes = in_bytes + (info.numel() + hw.numel() + sc.numel()) * 4
         self.d2h_bytes = n * 4
         # the exponents this step ran with (a captured graph keeps those of its capture)
         return (slot, B, n, scale, args, dict(eng.exp))
@@ -232,9 +327,9 @@ class Detector:
     def _step(self, slot, args, B):
         eng, st = self._engines[slot], self._slots[slot]
         if self.use_graph:
-            eng.detect_graphed(*args, rec=st["d_rec"])
+            eng.detect_graphed(*args[:4], rec=st["d_rec"], extents=args[4])
         else:
-            o = eng.forward(args[0], args[1])
+            o = eng.forward(args[0], args[1], extents=args[4])
             eng.detect_tail(o, B, args[2], args[3], rec=st["d_rec"])
 
     def _collect(self, handle):

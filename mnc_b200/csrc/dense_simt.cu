@@ -114,10 +114,20 @@ __global__ void __launch_bounds__(256)
 splitk_reduce_kernel(const float* __restrict__ partial, int splits, long long split_stride,
                      long long rows, int cols, const float* __restrict__ bias, int relu,
                      int out_mode, void* out0, void* out1, long long out_row_stride,
-                     int out_ch_offset, int vec) {
+                     int out_ch_offset, int vec, const int* __restrict__ img_hw, int level, int H,
+                     int W) {
   const int c4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
   if (c4 >= cols) return;
   for (long long r = blockIdx.y; r < rows; r += gridDim.y) {
+    // conv launches of mixed-size batches: row r is pixel (b, y, x); outside image b -> zeros
+    bool inside = true;
+    if (img_hw != nullptr) {
+      const long long hw = static_cast<long long>(H) * W;
+      const int b = static_cast<int>(r / hw), pr = static_cast<int>(r - b * hw);
+      const int m = (1 << level) - 1;
+      inside = pr / W < ((__ldg(img_hw + 2 * b) + m) >> level) &&
+               pr % W < ((__ldg(img_hw + 2 * b + 1) + m) >> level);
+    }
     float v[4] = {0.f, 0.f, 0.f, 0.f};
     const float* p = partial + r * cols + c4;
     if (vec) {
@@ -137,6 +147,7 @@ splitk_reduce_kernel(const float* __restrict__ partial, int splits, long long sp
     for (int e = 0; e < 4; ++e) {
       if (bias && c4 + e < cols) v[e] += __ldg(bias + c4 + e);
       if (relu) v[e] = fmaxf(v[e], 0.f);
+      if (!inside) v[e] = 0.f;
     }
     const long long o = r * out_row_stride + out_ch_offset + c4;
     if (out_mode == 0) {
@@ -413,11 +424,15 @@ extern "C" int mnc_igemm_simt(const void* a_hi, const void* a_lo, int batch, int
   return check_launch();
 }
 
-extern "C" int mnc_splitk_reduce(const float* partial, int splits, long long split_stride,
-                                 long long rows, int cols, const float* bias, int relu,
-                                 int out_mode, void* out0, void* out1, long long out_row_stride,
-                                 int out_ch_offset, void* stream) {
+extern "C" int mnc_splitk_reduce2(const float* partial, int splits, long long split_stride,
+                                  long long rows, int cols, const float* bias, int relu,
+                                  int out_mode, void* out0, void* out1, long long out_row_stride,
+                                  int out_ch_offset, const int* img_hw, int level, int H, int W,
+                                  void* stream) {
   if (rows <= 0 || cols <= 0) return MNC_OK;
+  if (img_hw != nullptr && (level < 0 || level > 16 || H <= 0 || W <= 0 ||
+                            rows % (static_cast<long long>(H) * W) != 0))
+    return MNC_ERR_ARG;
   const int vec = (cols % 4 == 0) && (split_stride % 4 == 0) && (out_row_stride % 4 == 0) &&
                   (out_ch_offset % 4 == 0) && (reinterpret_cast<uintptr_t>(partial) % 16 == 0) &&
                   (reinterpret_cast<uintptr_t>(out0) % 16 == 0) &&
@@ -427,8 +442,16 @@ extern "C" int mnc_splitk_reduce(const float* partial, int splits, long long spl
   dim3 grid((tx + block - 1) / block, static_cast<unsigned>(rows < 32768 ? rows : 32768));
   splitk_reduce_kernel<<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(
       partial, splits, split_stride, rows, cols, bias, relu, out_mode, out0, out1, out_row_stride,
-      out_ch_offset, vec);
+      out_ch_offset, vec, img_hw, level, H, W);
   return check_launch();
+}
+
+extern "C" int mnc_splitk_reduce(const float* partial, int splits, long long split_stride,
+                                 long long rows, int cols, const float* bias, int relu,
+                                 int out_mode, void* out0, void* out1, long long out_row_stride,
+                                 int out_ch_offset, void* stream) {
+  return mnc_splitk_reduce2(partial, splits, split_stride, rows, cols, bias, relu, out_mode, out0,
+                            out1, out_row_stride, out_ch_offset, nullptr, 0, 1, 1, stream);
 }
 
 extern "C" int mnc_conv1_1(const float* data_nchw, int batch, int H, int W, const float* weight,

@@ -57,7 +57,23 @@ struct IgemmArgs {
   long long split_stride;  // elements between split-K partial planes (fp32 mode)
   int vec_ok;              // 16-byte vector stores are aligned
   int tma_store;           // out_mode 0 only: epilogue stages tiles in smem and TMA-stores them
+  // Mixed-size batches: image b fills the top-left of the padded blob.  img_hw [batch][2] holds
+  // its size at input resolution; at this launch's trunk level (input halved `level` times,
+  // ceil mode) its extent is ((h + 2^level - 1) >> level, ...).  Pixels outside their image's
+  // extent are written as exact zeros and never enter a pool window or the published maximum.
+  // nullptr: every pixel of the blob is inside.
+  const int* img_hw;
+  int level;
+  int img_rows;            // > 0: tile "images" are single rows, image b = img / img_rows (conv1_1)
 };
+
+// Extent (rows, cols) of image b at p.level, clamped to the blob.
+__device__ __forceinline__ int2 img_extent(const IgemmArgs& p, int b, int H, int W) {
+  if (p.img_hw == nullptr) return make_int2(H, W);
+  const int m = (1 << p.level) - 1;
+  return make_int2(min(H, (__ldg(p.img_hw + 2 * b) + m) >> p.level),
+                   min(W, (__ldg(p.img_hw + 2 * b + 1) + m) >> p.level));
+}
 
 constexpr int kBlockM = 128;
 
@@ -170,7 +186,14 @@ __device__ __forceinline__ void run_epilogue(const IgemmArgs& p, const CUtensorM
     const uint32_t acc_phase = (local >> 1) & 1;
     const int h = h0 + row / TW;
     const int w = w0 + row % TW;
-    const bool valid = !tl.dummy && (h < p.H) && (w < p.W);
+    const bool inblob = !tl.dummy && (h < p.H) && (w < p.W);
+    // this tile's image and its row in it (conv1_1 runs one-row images), and the image's extent
+    const int eb = p.img_rows > 0 ? img / p.img_rows : img;
+    const int eh = p.img_rows > 0 ? img - eb * p.img_rows : h0;
+    const int2 ext = tl.dummy ? make_int2(0, 0)
+                              : img_extent(p, eb, p.img_rows > 0 ? p.img_rows : p.H, p.W);
+    const int hrow = eh + (h - h0);   // row within the image
+    const bool valid = inblob && hrow < ext.x && w < ext.y;
     const long long pix = (static_cast<long long>(img) * p.H + h) * p.W + w;
     ptx::mbar_wait(&tfull_bar[acc], acc_phase);
     ptx::tc_fence_after();
@@ -212,7 +235,9 @@ __device__ __forceinline__ void run_epilogue(const IgemmArgs& p, const CUtensorM
         float x[32];
 #pragma unroll
         for (int j = 0; j < 32; ++j) x[j] = __uint_as_float(r[j]);
-        if (!__all_sync(0xffffffffu, valid)) {   // ragged tile: rows outside the image never win
+        // ragged tile: rows outside the blob or outside this image's extent never win (a padded
+        // pixel's raw accumulator is not zero: it sees the image's edge through the 3x3 window)
+        if (!__all_sync(0xffffffffu, valid)) {
 #pragma unroll
           for (int j = 0; j < 32; ++j) x[j] = valid ? x[j] : -3.402823466e+38f;
         }
@@ -235,6 +260,9 @@ __device__ __forceinline__ void run_epilogue(const IgemmArgs& p, const CUtensorM
         const int chp = ch0 + part * 8;
         if (!tl.dummy && hp < Ho && wp < Wo && (h0 + hl) < p.H && (w0 + wl) < p.W &&
             chp < p.Cout) {
+          // pooled pixel inside the image's level+1 extent <=> its window's top-left pixel is
+          // inside the level extent; outside it the output is an exact zero
+          const bool pin = (h0 + hl) < ext.x && (w0 + wl) < ext.y;
           const long long ppix = (static_cast<long long>(img) * Ho + hp) * Wo + wp;
           const long long poff = ppix * p.out_pix_stride + p.out_ch_offset + chp;
           float bv[8];
@@ -252,6 +280,7 @@ __device__ __forceinline__ void run_epilogue(const IgemmArgs& p, const CUtensorM
           for (int j = 0; j < 8; ++j) {
             m[j] = m[j] * asc + bv[j];
             if (p.relu) m[j] = fmaxf(m[j], 0.f);
+            m[j] = pin ? m[j] : 0.f;
             if (chp + j < p.Cout) amx = fmaxf(amx, fabsf(m[j]));   // max |pooled output|
           }
           if (p.out_mode == 5) {
@@ -334,6 +363,10 @@ __device__ __forceinline__ void run_epilogue(const IgemmArgs& p, const CUtensorM
                 x0 = fmaxf(x0, 0.f);
                 x1 = fmaxf(x1, 0.f);
               }
+              if (!valid) {   // outside the image: exact zeros (TMA clips rows outside the blob)
+                x0 = 0.f;
+                x1 = 0.f;
+              }
               mx = fmaxf(mx, fmaxf(fabsf(x0), fabsf(x1)));
               if (tri) {
                 const Tri2 tr = tri_pack2(x0, x1, p.out_scale);
@@ -378,15 +411,15 @@ __device__ __forceinline__ void run_epilogue(const IgemmArgs& p, const CUtensorM
           ptx::tma_store_commit();
         }
         ++chunk_ctr;
-      } else if (valid && ch0 < p.Cout) {
+      } else if (inblob && ch0 < p.Cout) {
         float v[32];
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           float x = __uint_as_float(r[j]) * asc;
           if (p.bias != nullptr && ch0 + j < p.Cout) x += __ldg(p.bias + ch0 + j);
           if (p.relu) x = fmaxf(x, 0.f);
-          v[j] = x;
-          if (ch0 + j < p.Cout) amx = fmaxf(amx, fabsf(x));
+          v[j] = valid ? x : 0.f;   // outside the image: exact zeros
+          if (ch0 + j < p.Cout) amx = fmaxf(amx, fabsf(v[j]));
         }
         const bool fullchunk = (ch0 + 32 <= p.Cout) && p.vec_ok;
         if (p.out_mode == 0) {
@@ -1340,16 +1373,19 @@ extern "C" int mnc_igemm_set_block_k(int bk) {
 // exponent scale `out_scale`; 2 and 5 apply the fused 2x2 ceil-mode max pool.  acc_scale turns the
 // accumulator into the true value (2^-(ea+ew) for tri-plane operands, 1 otherwise).  amax
 // (optional, device) receives atomicMax(|output|) as float bits.
-extern "C" int mnc_igemm_tc2(int in_fmt, const void* a0, const void* a1, const void* a2, int batch,
+// img_hw (optional, device int32 [batch][2]) + level: per-image extents of a mixed-size batch
+// (IgemmArgs::img_hw); nullptr = the whole blob.
+extern "C" int mnc_igemm_tc3(int in_fmt, const void* a0, const void* a1, const void* a2, int batch,
                              int H, int W, int Cin, const void* w0, const void* w1, const void* w2,
                              int Cout, int taps, const float* bias, int relu, int out_mode,
                              void* out0, void* out1, void* out2, long long out_pix_stride,
                              int out_ch_offset, int split_k, long long split_stride, int bn,
                              int max_ctas, float acc_scale, float out_scale, unsigned int* amax,
-                             void* stream_) {
+                             const int* img_hw, int level, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   if (Cin % 64 != 0 || (taps != 1 && taps != 9) || batch <= 0 || H <= 0 || W <= 0 || Cout <= 0)
     return MNC_ERR_ARG;
+  if (level < 0 || level > 16) return MNC_ERR_ARG;
   if (in_fmt != 0 && in_fmt != 1) return MNC_ERR_ARG;
   if (out_mode != 0 && out_mode != 1 && out_mode != 2 && out_mode != 3 && out_mode != 4 && out_mode != 5)
     return MNC_ERR_ARG;
@@ -1403,6 +1439,9 @@ extern "C" int mnc_igemm_tc2(int in_fmt, const void* a0, const void* a1, const v
   a.acc_scale = acc_scale;
   a.out_scale = out_scale;
   a.amax = amax;
+  a.img_hw = img_hw;
+  a.level = level;
+  a.img_rows = 0;
   const int vec = (out_mode == 1) ? 4 : 8;
   a.vec_ok = (out_pix_stride % vec == 0) && (out_ch_offset % vec == 0) &&
              (reinterpret_cast<uintptr_t>(out0) % 16 == 0) &&
@@ -1492,6 +1531,18 @@ extern "C" int mnc_igemm_tc2(int in_fmt, const void* a0, const void* a1, const v
 #undef MNC_LAUNCH_PM
 }
 
+extern "C" int mnc_igemm_tc2(int in_fmt, const void* a0, const void* a1, const void* a2, int batch,
+                             int H, int W, int Cin, const void* w0, const void* w1, const void* w2,
+                             int Cout, int taps, const float* bias, int relu, int out_mode,
+                             void* out0, void* out1, void* out2, long long out_pix_stride,
+                             int out_ch_offset, int split_k, long long split_stride, int bn,
+                             int max_ctas, float acc_scale, float out_scale, unsigned int* amax,
+                             void* stream_) {
+  return mnc_igemm_tc3(in_fmt, a0, a1, a2, batch, H, W, Cin, w0, w1, w2, Cout, taps, bias, relu,
+                       out_mode, out0, out1, out2, out_pix_stride, out_ch_offset, split_k,
+                       split_stride, bn, max_ctas, acc_scale, out_scale, amax, nullptr, 0, stream_);
+}
+
 // Split-bf16 operands, outputs 0 / 1 / 2 (the round-1 entry point; kept for its callers).
 extern "C" int mnc_igemm_tc(const void* a_hi, const void* a_lo, int batch, int H, int W, int Cin,
                             const void* w_hi, const void* w_lo, int Cout, int taps,
@@ -1507,9 +1558,11 @@ extern "C" int mnc_igemm_tc(const void* a_hi, const void* a_lo, int batch, int H
 // plane of weight.reshape(64, 27) (k = c*9 + ky*3 + kx), columns 27..31 zero.
 // out_mode 0: split-bf16 planes (out0 = hi, out1 = lo); 4: tri-plane (out0 = fp16, out1 = e4m3
 // residual, out2 = e4m3 copy) scaled by out_scale.  amax (optional, device): atomicMax(|output|).
-extern "C" int mnc_conv1_1_tc2(const float* data_nchw, int batch, int H, int W, const void* w_stacked,
+// img_hw (optional, device int32 [batch][2]): per-image sizes of a mixed-size batch; output pixels
+// outside their image are written as zeros.
+extern "C" int mnc_conv1_1_tc3(const float* data_nchw, int batch, int H, int W, const void* w_stacked,
                                const float* bias, int out_mode, void* out0, void* out1, void* out2,
-                               float out_scale, unsigned int* amax, void* stream_) {
+                               float out_scale, unsigned int* amax, const int* img_hw, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   if (batch <= 0 || H <= 0 || W <= 0 || (out_mode != 0 && out_mode != 4)) return MNC_ERR_ARG;
   if ((reinterpret_cast<uintptr_t>(out0) | reinterpret_cast<uintptr_t>(out1) |
@@ -1543,6 +1596,9 @@ extern "C" int mnc_conv1_1_tc2(const float* data_nchw, int batch, int H, int W, 
   a.acc_scale = 1.0f;
   a.out_scale = out_scale;
   a.amax = amax;
+  a.img_hw = img_hw;
+  a.level = 0;
+  a.img_rows = H;
   CUtensorMap tb, to_hi, to_lo, to_x;
   int rc;
   const int eb = (out_mode == 4) ? 1 : 2;
@@ -1559,6 +1615,13 @@ extern "C" int mnc_conv1_1_tc2(const float* data_nchw, int batch, int H, int W, 
   conv1_1_tc_kernel<<<grid, kC11Threads, kC11Smem, stream>>>(data_nchw, batch, H, W, tb, to_hi, to_lo,
                                                              to_x, a);
   return cudaGetLastError() == cudaSuccess ? MNC_OK : MNC_ERR_CUDA;
+}
+
+extern "C" int mnc_conv1_1_tc2(const float* data_nchw, int batch, int H, int W, const void* w_stacked,
+                               const float* bias, int out_mode, void* out0, void* out1, void* out2,
+                               float out_scale, unsigned int* amax, void* stream_) {
+  return mnc_conv1_1_tc3(data_nchw, batch, H, W, w_stacked, bias, out_mode, out0, out1, out2,
+                         out_scale, amax, nullptr, stream_);
 }
 
 extern "C" int mnc_conv1_1_tc(const float* data_nchw, int batch, int H, int W, const void* w_stacked,

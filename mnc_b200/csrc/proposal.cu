@@ -79,7 +79,8 @@ __global__ void rpn_decode_kernel(const float* __restrict__ cls, long long cls_i
                                   const float* __restrict__ im_info, int H, int W, int feat_stride,
                                   float min_size, int apply_softmax, const Anchors anchors,
                                   float* __restrict__ proposals, float* __restrict__ scores,
-                                  unsigned char* __restrict__ valid) {
+                                  unsigned char* __restrict__ valid, const int* __restrict__ img_hw,
+                                  int level) {
   const int A = 9;
   const int total = H * W * A;
   const int img = blockIdx.y;
@@ -116,7 +117,13 @@ __global__ void rpn_decode_kernel(const float* __restrict__ cls, long long cls_i
   const long long oidx = static_cast<long long>(img) * total + t;
   *reinterpret_cast<float4*>(proposals + oidx * 4) = make_float4(o[0], o[1], o[2], o[3]);
   scores[oidx] = score;
-  valid[oidx] = (ws >= ms && hs >= ms) ? 1 : 0;
+  // mixed-size batch: anchors of the padded map outside this image's extent take no part
+  bool inside = true;
+  if (img_hw != nullptr) {
+    const int m = (1 << level) - 1;
+    inside = y < ((__ldg(img_hw + 2 * img) + m) >> level) && x < ((__ldg(img_hw + 2 * img + 1) + m) >> level);
+  }
+  valid[oidx] = (inside && ws >= ms && hs >= ms) ? 1 : 0;
 }
 
 // rois[img][k] = [batch_index, sorted_boxes[img][keep[img][k]]], zero rows past num_keep.
@@ -297,12 +304,13 @@ extern "C" int mnc_generate_anchors(float* out36) {
   return MNC_OK;
 }
 
-extern "C" int mnc_rpn_decode(const float* cls, long long cls_img_stride, long long cls_ch_stride,
-                              long long cls_pix_stride, const float* bbox, long long bb_img_stride,
-                              long long bb_ch_stride, long long bb_pix_stride,
-                              const float* im_info, int batch, int H, int W, int feat_stride,
-                              float min_size, int apply_softmax, float* proposals, float* scores,
-                              unsigned char* valid, void* stream) {
+extern "C" int mnc_rpn_decode2(const float* cls, long long cls_img_stride, long long cls_ch_stride,
+                               long long cls_pix_stride, const float* bbox, long long bb_img_stride,
+                               long long bb_ch_stride, long long bb_pix_stride,
+                               const float* im_info, int batch, int H, int W, int feat_stride,
+                               float min_size, int apply_softmax, float* proposals, float* scores,
+                               unsigned char* valid, const int* img_hw, int level, void* stream) {
+  if (level < 0 || level > 16) return MNC_ERR_ARG;
   Anchors an;
   double a[9][4];
   generate_anchors_host(a);
@@ -313,8 +321,19 @@ extern "C" int mnc_rpn_decode(const float* cls, long long cls_img_stride, long l
   rpn_decode_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
       cls, cls_img_stride, cls_ch_stride, cls_pix_stride, bbox, bb_img_stride, bb_ch_stride,
       bb_pix_stride, im_info, H, W, feat_stride, min_size, apply_softmax, an, proposals, scores,
-      valid);
+      valid, img_hw, level);
   return check_launch();
+}
+
+extern "C" int mnc_rpn_decode(const float* cls, long long cls_img_stride, long long cls_ch_stride,
+                              long long cls_pix_stride, const float* bbox, long long bb_img_stride,
+                              long long bb_ch_stride, long long bb_pix_stride,
+                              const float* im_info, int batch, int H, int W, int feat_stride,
+                              float min_size, int apply_softmax, float* proposals, float* scores,
+                              unsigned char* valid, void* stream) {
+  return mnc_rpn_decode2(cls, cls_img_stride, cls_ch_stride, cls_pix_stride, bbox, bb_img_stride,
+                         bb_ch_stride, bb_pix_stride, im_info, batch, H, W, feat_stride, min_size,
+                         apply_softmax, proposals, scores, valid, nullptr, 0, stream);
 }
 
 extern "C" int mnc_write_rois(const float* sorted_boxes, int n_sorted, const int* keep,

@@ -634,18 +634,28 @@ __device__ __forceinline__ void st_feat4(void* const (&pl)[3], long long off, co
 template <int SUB, bool TRI>
 __global__ void __launch_bounds__(256, 4)
 roi_warp_split_kernel(const float* __restrict__ feat, int C, int H, int W,
-                      const float* __restrict__ rois, float spatial_scale, const RoiOut o) {
+                      const float* __restrict__ rois, float spatial_scale, const RoiOut o,
+                      const int* __restrict__ img_hw, int level) {
   constexpr int P = 14 * SUB;
   constexpr int NS = 2 * SUB * P;  // samples handled by this CTA
   __shared__ SampleTab tab[NS];
   const int r = blockIdx.x;
   const int t = blockIdx.y;  // rows 2t, 2t+1 of the 14x14 grid
   const RoiGeom g = roi_geom(rois + static_cast<long long>(r) * 5, spatial_scale, P, P);
+  // mixed-size batch: samples are bounded and clamped by the extent of the RoI's image (the row
+  // stride stays the blob's W); the extent is clamped to [1, map] so that no sample can land
+  // outside the map even for an invalid (zero) size
+  int He = H, We = W;
+  if (img_hw != nullptr) {
+    const int m = (1 << level) - 1;
+    He = max(1, min(H, (__ldg(img_hw + 2 * g.level) + m) >> level));
+    We = max(1, min(W, (__ldg(img_hw + 2 * g.level + 1) + m) >> level));
+  }
   for (int i = threadIdx.x; i < NS; i += blockDim.x) {
     const int sr = i / P, pw = i - sr * P;
     const int ph = 2 * t * SUB + sr;
-    const AxisTap th = axis_tap(__fadd_rn(g.start_h, __fmul_rn(static_cast<float>(ph), g.bin_h)), H);
-    const AxisTap tw = axis_tap(__fadd_rn(g.start_w, __fmul_rn(static_cast<float>(pw), g.bin_w)), W);
+    const AxisTap th = axis_tap(__fadd_rn(g.start_h, __fmul_rn(static_cast<float>(ph), g.bin_h)), He);
+    const AxisTap tw = axis_tap(__fadd_rn(g.start_w, __fmul_rn(static_cast<float>(pw), g.bin_w)), We);
     const bool ok = th.ok && tw.ok;
     SampleTab e;
     e.off[0] = ok ? (th.lo * W + tw.lo) * C : 0;
@@ -1268,12 +1278,16 @@ extern "C" int mnc_roi_warp_set_walk(int on) {
   return prev;
 }
 
-extern "C" int mnc_roi_warp_split(const float* feat_nhwc, int C, int H, int W, const float* rois,
-                                  int R, int sub, float spatial_scale, void* o14_hi, void* o14_lo,
-                                  void* o7_hi, void* o7_lo, void* stream) {
+// img_hw (optional, device int32 [batch][2]) + level: per-image extents of a mixed-size batch;
+// the A/B kernel forms (set_walk / set_rows) do not take them.
+extern "C" int mnc_roi_warp_split2(const float* feat_nhwc, int C, int H, int W, const float* rois,
+                                   int R, int sub, float spatial_scale, void* o14_hi, void* o14_lo,
+                                   void* o7_hi, void* o7_lo, const int* img_hw, int level,
+                                   void* stream) {
   if (R <= 0) return MNC_OK;
   if (C % 4 != 0 || (sub != 1 && sub != 2) || (reinterpret_cast<uintptr_t>(feat_nhwc) & 15))
     return MNC_ERR_ARG;
+  if (img_hw != nullptr && (level < 0 || level > 16 || g_roi_walk || g_roi_rows)) return MNC_ERR_ARG;
   auto s = static_cast<cudaStream_t>(stream);
   if (g_roi_walk) {
     dim3 wgrid(R, 4);
@@ -1299,20 +1313,30 @@ extern "C" int mnc_roi_warp_split(const float* feat_nhwc, int C, int H, int W, c
   }
   dim3 grid(R, 7);
   if (sub == 2)
-    roi_warp_split_kernel<2, false><<<grid, 256, 0, s>>>(feat_nhwc, C, H, W, rois, spatial_scale, o);
+    roi_warp_split_kernel<2, false><<<grid, 256, 0, s>>>(feat_nhwc, C, H, W, rois, spatial_scale, o,
+        img_hw, level);
   else
-    roi_warp_split_kernel<1, false><<<grid, 256, 0, s>>>(feat_nhwc, C, H, W, rois, spatial_scale, o);
+    roi_warp_split_kernel<1, false><<<grid, 256, 0, s>>>(feat_nhwc, C, H, W, rois, spatial_scale, o,
+        img_hw, level);
   return check_launch();
 }
 
+extern "C" int mnc_roi_warp_split(const float* feat_nhwc, int C, int H, int W, const float* rois,
+                                  int R, int sub, float spatial_scale, void* o14_hi, void* o14_lo,
+                                  void* o7_hi, void* o7_lo, void* stream) {
+  return mnc_roi_warp_split2(feat_nhwc, C, H, W, rois, R, sub, spatial_scale, o14_hi, o14_lo, o7_hi,
+                             o7_lo, nullptr, 0, stream);
+}
+
 // Same, writing tri-plane outputs (fp16 value, e4m3 residual, e4m3 copy) scaled by `scale` = 2^exp.
-extern "C" int mnc_roi_warp_tri(const float* feat_nhwc, int C, int H, int W, const float* rois,
-                                int R, int sub, float spatial_scale, float scale, void* o14_h,
-                                void* o14_l, void* o14_c, void* o7_h, void* o7_l, void* o7_c,
-                                void* stream) {
+extern "C" int mnc_roi_warp_tri2(const float* feat_nhwc, int C, int H, int W, const float* rois,
+                                 int R, int sub, float spatial_scale, float scale, void* o14_h,
+                                 void* o14_l, void* o14_c, void* o7_h, void* o7_l, void* o7_c,
+                                 const int* img_hw, int level, void* stream) {
   if (R <= 0) return MNC_OK;
   if (C % 4 != 0 || (sub != 1 && sub != 2) || (reinterpret_cast<uintptr_t>(feat_nhwc) & 15))
     return MNC_ERR_ARG;
+  if (img_hw != nullptr && (level < 0 || level > 16 || g_roi_rows)) return MNC_ERR_ARG;
   auto s = static_cast<cudaStream_t>(stream);
   RoiOut o;
   o.p14[0] = o14_h; o.p14[1] = o14_l; o.p14[2] = o14_c;
@@ -1324,10 +1348,20 @@ extern "C" int mnc_roi_warp_tri(const float* feat_nhwc, int C, int H, int W, con
   }
   dim3 grid(R, 7);
   if (sub == 2)
-    roi_warp_split_kernel<2, true><<<grid, 256, 0, s>>>(feat_nhwc, C, H, W, rois, spatial_scale, o);
+    roi_warp_split_kernel<2, true><<<grid, 256, 0, s>>>(feat_nhwc, C, H, W, rois, spatial_scale, o,
+        img_hw, level);
   else
-    roi_warp_split_kernel<1, true><<<grid, 256, 0, s>>>(feat_nhwc, C, H, W, rois, spatial_scale, o);
+    roi_warp_split_kernel<1, true><<<grid, 256, 0, s>>>(feat_nhwc, C, H, W, rois, spatial_scale, o,
+        img_hw, level);
   return check_launch();
+}
+
+extern "C" int mnc_roi_warp_tri(const float* feat_nhwc, int C, int H, int W, const float* rois,
+                                int R, int sub, float spatial_scale, float scale, void* o14_h,
+                                void* o14_l, void* o14_c, void* o7_h, void* o7_l, void* o7_c,
+                                void* stream) {
+  return mnc_roi_warp_tri2(feat_nhwc, C, H, W, rois, R, sub, spatial_scale, scale, o14_h, o14_l,
+                           o14_c, o7_h, o7_l, o7_c, nullptr, 0, stream);
 }
 
 extern "C" int mnc_roi_pool_nchw(const float* feat, int C, int H, int W, const float* rois, int R,

@@ -41,14 +41,25 @@ tri_to_f32_kernel(const __half* __restrict__ h, const uint8_t* __restrict__ l, l
   }
 }
 
+// Is conv output row `row` (= pixel (b, y, x) of a [B][H][W] map) inside its image's extent at
+// trunk level `level`?  img_hw: device int32 [B][2] input-resolution sizes (mixed-size batches).
+__device__ __forceinline__ bool row_in_image(const int* img_hw, int level, int H, int W, long long row) {
+  if (img_hw == nullptr) return true;
+  const long long hw = static_cast<long long>(H) * W;
+  const int b = static_cast<int>(row / hw);
+  const int r = static_cast<int>(row - b * hw);
+  const int m = (1 << level) - 1;
+  return r / W < ((__ldg(img_hw + 2 * b) + m) >> level) && r % W < ((__ldg(img_hw + 2 * b + 1) + m) >> level);
+}
+
 // out[row][ch_offset + col] = act(sum_s partial[s][row][col] + bias[col]) as tri-plane; one thread
-// per 4 columns.
+// per 4 columns.  Rows outside their image (img_hw, conv launches of mixed-size batches) are zeros.
 __global__ void __launch_bounds__(256)
 splitk_reduce_tri_kernel(const float* __restrict__ partial, int splits, long long split_stride,
                          long long rows, int cols, const float* __restrict__ bias, int relu,
                          float scale, __half* __restrict__ h, uint8_t* __restrict__ l,
                          uint8_t* __restrict__ c, long long out_row_stride, int out_ch_offset,
-                         unsigned int* amax) {
+                         unsigned int* amax, const int* __restrict__ img_hw, int level, int H, int W) {
   const int c4 = cols >> 2;
   float amx = 0.f;
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < rows * c4;
@@ -68,6 +79,7 @@ splitk_reduce_tri_kernel(const float* __restrict__ partial, int splits, long lon
     if (relu) {
       acc.x = fmaxf(acc.x, 0.f); acc.y = fmaxf(acc.y, 0.f); acc.z = fmaxf(acc.z, 0.f); acc.w = fmaxf(acc.w, 0.f);
     }
+    if (!row_in_image(img_hw, level, H, W, row)) acc = make_float4(0.f, 0.f, 0.f, 0.f);
     amx = fmaxf(amx, fmaxf(fmaxf(fabsf(acc.x), fabsf(acc.y)), fmaxf(fabsf(acc.z), fabsf(acc.w))));
     st_tri4(h, l, c, row * out_row_stride + out_ch_offset + col, acc, scale);
   }
@@ -138,20 +150,34 @@ extern "C" int mnc_tri_to_f32(const void* h, const void* l, long long n, float i
   return tri_check_launch();
 }
 
-extern "C" int mnc_splitk_reduce_tri(const float* partial, int splits, long long split_stride,
-                                     long long rows, int cols, const float* bias, int relu,
-                                     float scale, void* h, void* l, void* c,
-                                     long long out_row_stride, int out_ch_offset,
-                                     unsigned int* amax, void* stream) {
+extern "C" int mnc_splitk_reduce_tri2(const float* partial, int splits, long long split_stride,
+                                      long long rows, int cols, const float* bias, int relu,
+                                      float scale, void* h, void* l, void* c,
+                                      long long out_row_stride, int out_ch_offset,
+                                      unsigned int* amax, const int* img_hw, int level, int H,
+                                      int W, void* stream) {
   if (rows <= 0 || cols <= 0) return MNC_OK;
+  if (img_hw != nullptr && (level < 0 || level > 16 || H <= 0 || W <= 0 ||
+                            rows % (static_cast<long long>(H) * W) != 0))
+    return MNC_ERR_ARG;
   if (cols % 4 != 0 || split_stride % 4 != 0 || out_row_stride % 4 != 0 || out_ch_offset % 4 != 0 ||
       reinterpret_cast<uintptr_t>(partial) % 16 != 0 ||
       (bias != nullptr && reinterpret_cast<uintptr_t>(bias) % 16 != 0))
     return MNC_ERR_ARG;
   splitk_reduce_tri_kernel<<<tri_grid(rows * (cols / 4), 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       partial, splits, split_stride, rows, cols, bias, relu, scale, static_cast<__half*>(h),
-      static_cast<uint8_t*>(l), static_cast<uint8_t*>(c), out_row_stride, out_ch_offset, amax);
+      static_cast<uint8_t*>(l), static_cast<uint8_t*>(c), out_row_stride, out_ch_offset, amax,
+      img_hw, level, H, W);
   return tri_check_launch();
+}
+
+extern "C" int mnc_splitk_reduce_tri(const float* partial, int splits, long long split_stride,
+                                     long long rows, int cols, const float* bias, int relu,
+                                     float scale, void* h, void* l, void* c,
+                                     long long out_row_stride, int out_ch_offset,
+                                     unsigned int* amax, void* stream) {
+  return mnc_splitk_reduce_tri2(partial, splits, split_stride, rows, cols, bias, relu, scale, h, l, c,
+                                out_row_stride, out_ch_offset, amax, nullptr, 0, 1, 1, stream);
 }
 
 extern "C" int mnc_mask_pool_tri(const void* f_h, const void* f_l, const float* mask14, int R, int C,

@@ -121,9 +121,11 @@ def fc_weight_to_tri(w, chw=None):
 
 def igemm2(a, batch, H, W, cin, w, cout, taps, bias=None, relu=False, out=None, out_f32=None,
            out_pix_stride=None, out_ch_offset=0, split_k=1, split_stride=0, bn=0, max_ctas=0,
-           pool=False, out_exp=0, amax=None):
+           pool=False, out_exp=0, amax=None, img_hw=None, level=0):
     """General tensor-core launch (mnc_igemm_tc2).  a / w: split bf16 tensors ([2, ...]) or Tri;
-    out: split bf16 tensor, or Tri (written with exponent out_exp), or out_f32."""
+    out: split bf16 tensor, or Tri (written with exponent out_exp), or out_f32.
+    img_hw: device int32 (batch, 2) image sizes of a mixed-size batch, `level` pools below the
+    input (mnc_igemm_tc3): pixels outside their image come out as zeros."""
     tri_in = isinstance(a, Tri)
     assert tri_in == isinstance(w, Tri)
     if tri_in:
@@ -144,14 +146,17 @@ def igemm2(a, batch, H, W, cin, w, cout, taps, bias=None, relu=False, out=None, 
         ev0 = torch.cuda.Event(enable_timing=True)
         ev1 = torch.cuda.Event(enable_timing=True)
         ev0.record()
-    rc = lib.mnc_igemm_tc2(c_int(int(tri_in)), ptr(ap[0]), ptr(ap[1]), ptr(ap[2]), c_int(batch),
-                           c_int(H), c_int(W), c_int(cin), ptr(wp[0]), ptr(wp[1]), ptr(wp[2]),
-                           c_int(cout), c_int(taps), ptr(bias), c_int(int(relu)), c_int(mode),
-                           ptr(op[0]), ptr(op[1]), ptr(op[2]), c_ll(stride), c_int(out_ch_offset),
-                           c_int(split_k), c_ll(split_stride), c_int(bn), c_int(max_ctas),
-                           ctypes.c_float(acc_scale), ctypes.c_float(2.0 ** out_exp), ptr(amax),
-                           cur_stream())
-    check(rc, "mnc_igemm_tc2")
+    args = (c_int(int(tri_in)), ptr(ap[0]), ptr(ap[1]), ptr(ap[2]), c_int(batch),
+            c_int(H), c_int(W), c_int(cin), ptr(wp[0]), ptr(wp[1]), ptr(wp[2]),
+            c_int(cout), c_int(taps), ptr(bias), c_int(int(relu)), c_int(mode),
+            ptr(op[0]), ptr(op[1]), ptr(op[2]), c_ll(stride), c_int(out_ch_offset),
+            c_int(split_k), c_ll(split_stride), c_int(bn), c_int(max_ctas),
+            ctypes.c_float(acc_scale), ctypes.c_float(2.0 ** out_exp), ptr(amax))
+    if img_hw is None:
+        check(lib.mnc_igemm_tc2(*args, cur_stream()), "mnc_igemm_tc2")
+    else:
+        check(lib.mnc_igemm_tc3(*args, ptr(img_hw_arg(img_hw, batch)), c_int(level), cur_stream()),
+              "mnc_igemm_tc3")
     if timer is not None:
         ev1.record()
         timer.records.append((ev0, ev1, 2.0 * batch * H * W * cout * taps * cin,
@@ -163,6 +168,16 @@ def igemm2(a, batch, H, W, cin, w, cout, taps, bias=None, relu=False, out=None, 
             flops=2.0 * batch * H * W * cout * taps * cin,
             bytes=4.0 * (batch * H * W * cin + cout * taps * cin + m_out * cout * max(split_k, 1))))
 
+
+
+def img_hw_arg(img_hw, batch):
+    """Per-image sizes of a mixed-size batch as the kernels read them: a contiguous device int32
+    (batch, 2) tensor (shape and type are checked here; the values are the caller's to validate,
+    engine.check_extents)."""
+    if not (img_hw.is_cuda and img_hw.dtype == torch.int32 and img_hw.is_contiguous()
+            and tuple(img_hw.shape) == (batch, 2)):
+        raise ValueError("img_hw must be a contiguous device int32 tensor of shape (%d, 2)" % batch)
+    return img_hw
 
 
 class KernelTimer:
@@ -237,6 +252,12 @@ def set_cluster(cl):
     cluster_size = cl
 
 
+def set_tma_store(on):
+    """A/B and test switch: out_mode 0 epilogues through shared memory + TMA store (default on)
+    or direct per-thread stores."""
+    check(lib.mnc_igemm_set_tma_store(c_int(int(on))), "mnc_igemm_set_tma_store")
+
+
 def set_halo_pair(on):
     """A/B: CTA pairs in the halo kernel's precision mode 1 (default on)."""
     check(lib.mnc_igemm_set_halo_pair(c_int(int(on))), "mnc_igemm_set_halo_pair")
@@ -248,16 +269,23 @@ def set_block_k(bk):
 
 
 def splitk_reduce(partial, splits, split_stride, rows, cols, bias=None, relu=False, out=None,
-                  out_f32=None, out_row_stride=None, out_ch_offset=0):
+                  out_f32=None, out_row_stride=None, out_ch_offset=0, img_hw=None, level=0,
+                  map_hw=None):
+    """img_hw / level / map_hw = (H, W): the rows are the pixels of a conv launch over a
+    (batch, H, W) map of a mixed-size batch; rows outside their image come out as zeros."""
     if out_f32 is not None:
         mode, o0, o1 = 1, out_f32, None
     else:
         mode, o0, o1 = 0, out[0], out[1]
     stride = out_row_stride if out_row_stride is not None else cols
-    rc = lib.mnc_splitk_reduce(ptr(partial), c_int(splits), c_ll(split_stride), c_ll(rows),
-                               c_int(cols), ptr(bias), c_int(int(relu)), c_int(mode), ptr(o0),
-                               ptr(o1), c_ll(stride), c_int(out_ch_offset), cur_stream())
-    check(rc, "mnc_splitk_reduce")
+    args = (ptr(partial), c_int(splits), c_ll(split_stride), c_ll(rows), c_int(cols), ptr(bias),
+            c_int(int(relu)), c_int(mode), ptr(o0), ptr(o1), c_ll(stride), c_int(out_ch_offset))
+    if img_hw is None:
+        check(lib.mnc_splitk_reduce(*args, cur_stream()), "mnc_splitk_reduce")
+    else:
+        H, W = map_hw
+        check(lib.mnc_splitk_reduce2(*args, ptr(img_hw_arg(img_hw, rows // (H * W))), c_int(level), c_int(H),
+                                     c_int(W), cur_stream()), "mnc_splitk_reduce2")
 
 
 def conv1_1(data, weight, bias, out):
@@ -277,8 +305,9 @@ def conv1_1_weight_to_tc(weight):
     return sp.reshape(128, 32).contiguous()
 
 
-def conv1_1_tc(data, w_stacked, bias, out, out_exp=0, amax=None):
-    """out: split bf16 [2, B, H, W, 64] or Tri (written with exponent out_exp)."""
+def conv1_1_tc(data, w_stacked, bias, out, out_exp=0, amax=None, img_hw=None):
+    """out: split bf16 [2, B, H, W, 64] or Tri (written with exponent out_exp).  img_hw: image
+    sizes of a mixed-size batch (device int32 (B, 2)); outputs outside an image are zeros."""
     b, c, H, W = data.shape
     assert c == 3 and data.dtype == torch.float32 and data.is_contiguous()
     assert w_stacked.dtype == torch.bfloat16 and tuple(w_stacked.shape) == (128, 32)
@@ -287,10 +316,12 @@ def conv1_1_tc(data, w_stacked, bias, out, out_exp=0, amax=None):
         mode, op = 4, (out.h, out.l, out.c)
     else:
         mode, op = 0, (out[0], out[1], None)
-    rc = lib.mnc_conv1_1_tc2(ptr(data), c_int(b), c_int(H), c_int(W), ptr(w_stacked), ptr(bias),
-                             c_int(mode), ptr(op[0]), ptr(op[1]), ptr(op[2]),
-                             ctypes.c_float(2.0 ** out_exp), ptr(amax), cur_stream())
-    check(rc, "mnc_conv1_1_tc2")
+    args = (ptr(data), c_int(b), c_int(H), c_int(W), ptr(w_stacked), ptr(bias), c_int(mode),
+            ptr(op[0]), ptr(op[1]), ptr(op[2]), ctypes.c_float(2.0 ** out_exp), ptr(amax))
+    if img_hw is None:
+        check(lib.mnc_conv1_1_tc2(*args, cur_stream()), "mnc_conv1_1_tc2")
+    else:
+        check(lib.mnc_conv1_1_tc3(*args, ptr(img_hw_arg(img_hw, b)), cur_stream()), "mnc_conv1_1_tc3")
 
 
 def maxpool2x2(a, batch, H, W, C, out):
@@ -336,11 +367,16 @@ def f32_to_tri(x, out, exp, amax=None):
 
 
 def splitk_reduce_tri(partial, splits, split_stride, rows, cols, out, out_exp, bias=None, relu=False,
-                      out_row_stride=None, out_ch_offset=0, amax=None):
+                      out_row_stride=None, out_ch_offset=0, amax=None, img_hw=None, level=0,
+                      map_hw=None):
     out.exp = int(out_exp)
     stride = out_row_stride if out_row_stride is not None else cols
-    rc = lib.mnc_splitk_reduce_tri(ptr(partial), c_int(splits), c_ll(split_stride), c_ll(rows),
-                                   c_int(cols), ptr(bias), c_int(int(relu)),
-                                   ctypes.c_float(2.0 ** out_exp), ptr(out.h), ptr(out.l), ptr(out.c),
-                                   c_ll(stride), c_int(out_ch_offset), ptr(amax), cur_stream())
-    check(rc, "mnc_splitk_reduce_tri")
+    args = (ptr(partial), c_int(splits), c_ll(split_stride), c_ll(rows), c_int(cols), ptr(bias),
+            c_int(int(relu)), ctypes.c_float(2.0 ** out_exp), ptr(out.h), ptr(out.l), ptr(out.c),
+            c_ll(stride), c_int(out_ch_offset), ptr(amax))
+    if img_hw is None:
+        check(lib.mnc_splitk_reduce_tri(*args, cur_stream()), "mnc_splitk_reduce_tri")
+    else:
+        H, W = map_hw
+        check(lib.mnc_splitk_reduce_tri2(*args, ptr(img_hw_arg(img_hw, rows // (H * W))), c_int(level),
+                                         c_int(H), c_int(W), cur_stream()), "mnc_splitk_reduce_tri2")

@@ -32,6 +32,7 @@ def _ceil_half(x):
 
 
 HALO_MAX_COUT = 128    # 3x3 convs with Cout <= 128 run the halo kernel
+C5_LEVEL = 4           # conv5_x, the RPN and the RoI features sit four 2x2 pools below the input
 
 # Largest max |value| * 2^exp a tri-plane tensor may reach before its exponent counts as stale.
 # Calibration puts the maximum in (2^11, 2^12].  fp16 itself saturates only at 65504, but the e4m3
@@ -45,6 +46,31 @@ RANGE_MAX = 2.0 ** 14
 def in_range(amax, exp):
     """Is a tensor whose max |value| is `amax` still carried accurately with exponent `exp`?"""
     return amax * 2.0 ** exp <= RANGE_MAX
+
+
+def level_extent(n, level):
+    """Rows (or columns) that an image of n input rows covers `level` 2x2 ceil-mode pools deeper:
+    ceil(n / 2^level), Caffe's chain of ceil-mode halvings (pooling_layer.cpp:90-93)."""
+    return (n + (1 << level) - 1) >> level
+
+
+def check_extents(extents, H, W, max_batch=None):
+    """Host validation of the per-image sizes of a mixed-size batch: an int (B, 2) array of
+    (rows, cols) at input resolution, each >= 1 and within the (H, W) blob.  Returns it as a
+    contiguous int32 CPU tensor.  Raises ValueError (nothing has been launched)."""
+    import numpy as np
+    e = np.asarray(extents.cpu() if isinstance(extents, torch.Tensor) else extents)
+    if e.ndim != 2 or e.shape[1] != 2 or e.shape[0] < 1:
+        raise ValueError("extents must have shape (B, 2), got %s" % (e.shape,))
+    if max_batch is not None and e.shape[0] > max_batch:
+        raise ValueError("%d images in one batch, at most %d" % (e.shape[0], max_batch))
+    if not np.issubdtype(e.dtype, np.integer):
+        raise ValueError("extents must be integers")
+    if (e < 1).any():
+        raise ValueError("every image extent must be at least 1 pixel: %s" % e.tolist())
+    if (e[:, 0] > H).any() or (e[:, 1] > W).any():
+        raise ValueError("image extents %s exceed the %dx%d blob" % (e.tolist(), H, W))
+    return torch.from_numpy(np.ascontiguousarray(e, dtype=np.int32))
 
 
 def pick_split_k(tiles_m, tiles_n, k_steps, sms, cluster=2, max_split=32, out_elems=0):
@@ -165,12 +191,24 @@ class MNCEngine:
         return dense.fc_weight_to_tri(w, chw) if self.tri else dense.fc_weight_to_split(w, chw)
 
     # ------------------------------------------------------------------ helpers
+    def _drop_graphs(self, old):
+        """Buffer `old` is being replaced by a larger one (a bigger blob or batch than any so far):
+        graphs captured over it would replay into freed memory, so they go (after the work queued
+        on them has finished)."""
+        graphs = getattr(self, "_graphs", None)
+        if old is None or not graphs:
+            return
+        if not torch.cuda.is_current_stream_capturing():
+            torch.cuda.synchronize(self.device)
+        graphs.clear()
+
     def _split_buf(self, key, *shape):
         t = self._buf.get(key)
         need = 1
         for s in shape:
             need *= s
         if t is None or t.numel() < 2 * need:
+            self._drop_graphs(t)
             t = torch.empty(2 * need, dtype=torch.bfloat16, device=self.device)
             self._buf[key] = t
         return t[:2 * need].view(2, *shape)
@@ -184,6 +222,7 @@ class MNCEngine:
             need *= s_
         t = self._buf.get("tri_" + key)
         if t is None or t.numel() < 4 * need:
+            self._drop_graphs(t)
             t = torch.empty(4 * need, dtype=torch.uint8, device=self.device)
             self._buf["tri_" + key] = t
         return dense.Tri(t[:2 * need].view(torch.float16).view(*shape), t[2 * need:3 * need].view(*shape),
@@ -240,13 +279,31 @@ class MNCEngine:
             out = step(*args, **kwargs)
         return out
 
-    def forward_checked(self, data, im_info, keep_intermediate=False):
+    def forward_checked(self, data, im_info, keep_intermediate=False, extents=None):
         """`forward` with the per-call range check of `run_checked`."""
-        return self.run_checked(self.forward, data, im_info, keep_intermediate)
+        return self.run_checked(self.forward, data, im_info, keep_intermediate, extents=extents)
 
-    def detect_checked(self, data, im_info, im_hw, im_scale):
+    def detect_checked(self, data, im_info, im_hw, im_scale, extents=None):
         """`detect` with the per-call range check of `run_checked`."""
-        return self.run_checked(self.detect, data, im_info, im_hw, im_scale)
+        return self.run_checked(self.detect, data, im_info, im_hw, im_scale, extents=extents)
+
+    def _extents(self, data, extents):
+        """The device int32 (B, 2) image sizes of a mixed-size batch (None: every image fills the
+        blob).  A host array is validated (check_extents) and uploaded; a device tensor is taken
+        as is -- checking its values would cost a host sync, so a caller passing device extents
+        must have validated them (the kernels clamp them to the map, but invalid sizes give wrong
+        results)."""
+        if extents is None:
+            return None
+        if self.impl != "tc" or not self.fuse_pool or self.conv1_1_tc is None:
+            raise NotImplementedError("mixed-size batches run on the tensor-core path with fused "
+                                      "pools and the tensor-core conv1_1 only")
+        B, _, H, W = data.shape
+        if not (isinstance(extents, torch.Tensor) and extents.is_cuda):
+            extents = check_extents(extents, H, W).to(self.device, non_blocking=True)
+        if extents.dtype != torch.int32 or tuple(extents.shape) != (B, 2):
+            raise ValueError("extents must be int32 of shape (%d, 2)" % B)
+        return extents.contiguous()
 
     def _f32_buf(self, key, *shape):
         t = self._buf.get(key)
@@ -254,6 +311,7 @@ class MNCEngine:
         for s in shape:
             need *= s
         if t is None or t.numel() < need:
+            self._drop_graphs(t)
             t = torch.empty(need, dtype=torch.float32, device=self.device)
             self._buf[key] = t
         return t[:need].view(*shape)
@@ -308,9 +366,10 @@ class MNCEngine:
         """Split-K factor of one tensor-core launch: see pick_split_k."""
         return pick_split_k(tiles_m, tiles_n, k_steps, self.sms, dense.cluster_size, max_split, out_elems)
 
-    def _conv(self, x, B, H, W, cin, wgt, cout, bias, out, key, pool=False):
+    def _conv(self, x, B, H, W, cin, wgt, cout, bias, out, key, pool=False, ext=None, level=0):
         """3x3 conv + bias + ReLU (+ fused 2x2 ceil-mode max pool) -> `out` (split-bf16 or Tri),
-        split-K when whole waves would idle."""
+        split-K when whole waves would idle.  ext / level: image sizes of a mixed-size batch and
+        the input's depth in pools (pixels outside an image come out as zeros)."""
         if self.impl != "tc":
             dense.igemm(x, B, H, W, cin, wgt, cout, 9, bias=bias, relu=True, out=out, impl=self.impl)
             return
@@ -322,7 +381,7 @@ class MNCEngine:
         if split == 1:
             def run(e, amax):
                 dense.igemm2(x, B, H, W, cin, wgt, cout, 9, bias=bias, relu=True, out=out, pool=pool,
-                             out_exp=e, amax=amax)
+                             out_exp=e, amax=amax, img_hw=ext, level=level)
             if tri_out:
                 self._scaled(key, run)
             else:
@@ -333,19 +392,25 @@ class MNCEngine:
         dense.igemm2(x, B, H, W, cin, wgt, cout, 9, out_f32=part, split_k=split, split_stride=M * cout)
         if tri_out:
             self._scaled(key, lambda e, amax: dense.splitk_reduce_tri(
-                part, split, M * cout, M, cout, out, e, bias=bias, relu=True, amax=amax))
+                part, split, M * cout, M, cout, out, e, bias=bias, relu=True, amax=amax,
+                img_hw=ext, level=level, map_hw=(H, W)))
         else:
-            dense.splitk_reduce(part, split, M * cout, M, cout, bias=bias, relu=True, out=out)
+            dense.splitk_reduce(part, split, M * cout, M, cout, bias=bias, relu=True, out=out,
+                                img_hw=ext, level=level, map_hw=(H, W))
 
     # ------------------------------------------------------------------ trunk
     def _conv_in_tri(self, cout):
         """Does the conv with `cout` output channels read tri-plane operands?"""
         return self.tri and (cout > HALO_MAX_COUT or self.halo_tri)
 
-    def trunk(self, data):
+    def trunk(self, data, extents=None):
         """conv1_1 .. conv5_3 (test.prototxt:19-387).  data fp32 (B,3,H,W) -> NHWC conv5_3 in the
-        format its consumers read (split bf16, or Tri when rpn_conv_3x3 takes tri-plane operands)."""
+        format its consumers read (split bf16, or Tri when rpn_conv_3x3 takes tri-plane operands).
+        extents: device int32 (B, 2) image sizes of a mixed-size batch (zero-padded blob); every
+        layer's output is then zero outside each image, as if it had run on that image alone."""
         B, _, H, W = data.shape
+        ext = self._extents(data, extents)
+        level = 0
         ch = self.arch["trunk"]
         big = B * H * W * max(ch[0], ch[1])
         cur = 0
@@ -360,9 +425,9 @@ class MNCEngine:
         if isinstance(x, dense.Tri):
             d = data.contiguous()
             self._scaled("conv1_1", lambda e, amax: dense.conv1_1_tc(
-                d, self.conv1_1_tc, self.conv1_1[1], x, out_exp=e, amax=amax))
+                d, self.conv1_1_tc, self.conv1_1[1], x, out_exp=e, amax=amax, img_hw=ext))
         elif self.conv1_1_tc is not None:
-            dense.conv1_1_tc(data.contiguous(), self.conv1_1_tc, self.conv1_1[1], x)
+            dense.conv1_1_tc(data.contiguous(), self.conv1_1_tc, self.conv1_1[1], x, img_hw=ext)
         else:
             dense.conv1_1(data, self.conv1_1[0], self.conv1_1[1], x)
         cin = ch[0]
@@ -384,8 +449,9 @@ class MNCEngine:
                     y = self._act_buf("conv5_3", B, Ho, Wo, cout, tri=nxt_tri, exp_key="conv5_3")
                 else:
                     y = self._pp_buf(nxt, nxt_tri, name, B, Ho, Wo, cout)
-                self._conv(x, B, H, W, cin, wgt, cout, bias, y, name, pool=fuse)
+                self._conv(x, B, H, W, cin, wgt, cout, bias, y, name, pool=fuse, ext=ext, level=level)
                 x, cur, cin, H, W = y, nxt, cout, Ho, Wo
+                level += int(fuse)
                 continue
             # un-fused pooling (SIMT cross-check path): split-bf16 only
             y = self._pp_buf(nxt, False, name, B, H, W, cout)
@@ -498,35 +564,45 @@ class MNCEngine:
             self.exp["roi_feat"] = dense.exp_for(amax, 12) if amax > 0 else 0
         return c5f
 
-    def rpn_rois(self, data, im_info, keep_intermediate=False):
+    def rpn_rois(self, data, im_info, keep_intermediate=False, extents=None):
         """test.prototxt:19-476: trunk, rpn_conv_3x3, rpn_cls_score | rpn_bbox_pred, softmax,
-        ProposalLayer.  -> conv5_3 (NHWC), H5, W5, fp32 conv5_3, rois (B*300,5), counts."""
+        ProposalLayer.  -> conv5_3 (NHWC), H5, W5, fp32 conv5_3, rois (B*300,5), counts.
+        extents: image sizes of a mixed-size batch (`trunk`); anchors outside an image take no
+        part in its proposals."""
         B = data.shape[0]
-        conv5_3, H5, W5 = self.trunk(data)
+        ext = self._extents(data, extents)
+        conv5_3, H5, W5 = self.trunk(data, ext)
         c5, r = self.c5, self.arch["rpn"]
         name, wgt, bias = self.convs[-1]
         rpn = self._act_buf("rpn", B, H5, W5, r, exp_key="rpn")     # consumer: the 54-wide head
-        self._conv(conv5_3, B, H5, W5, c5, wgt, r, bias, rpn, "rpn")
+        self._conv(conv5_3, B, H5, W5, c5, wgt, r, bias, rpn, "rpn", ext=ext, level=C5_LEVEL)
         rpn_out = self._f32_buf("rpn_out", B, H5, W5, 64)
         self._linear(rpn, B * H5 * W5, r, self.rpn_head[0], 54, self.rpn_head[1], False,
                      out_f32=rpn_out, out_stride=64, key="rpn_head")
         res = ops.proposals_from_rpn(rpn_out, None, im_info, B, H5, W5, "nhwc", True,
                                      pre_nms_top_n=PRE_NMS_TOP_N, post_nms_top_n=ROIS_PER_IMAGE,
                                      nms_thresh=RPN_NMS_THRESH, min_size=RPN_MIN_SIZE,
-                                     batch_index_mode=True, return_intermediate=keep_intermediate)
+                                     batch_index_mode=True, return_intermediate=keep_intermediate,
+                                     img_hw=ext, level=C5_LEVEL)
         rois = res[0].view(B * ROIS_PER_IMAGE, 5)
         return conv5_3, H5, W5, self.conv5_f32(conv5_3, B, H5, W5), rois, res[1], res, rpn_out
 
-    def roi_features(self, c5f, H5, W5, rois, sub, feat14, box7):
-        """ROIWarping (+ 28->14 pool when sub == 2) + 14->7 pool into the FC operand buffers."""
+    def roi_features(self, c5f, H5, W5, rois, sub, feat14, box7, extents=None):
+        """ROIWarping (+ 28->14 pool when sub == 2) + 14->7 pool into the FC operand buffers.
+        extents: image sizes of a mixed-size batch; a RoI samples its own image only."""
         if isinstance(feat14, dense.Tri):
-            ops.roi_warp_tri(c5f, self.c5, H5, W5, rois, sub, feat14, box7, self.exp["roi_feat"])
+            ops.roi_warp_tri(c5f, self.c5, H5, W5, rois, sub, feat14, box7, self.exp["roi_feat"],
+                             img_hw=extents, level=C5_LEVEL)
         else:
-            ops.roi_warp_split(c5f, self.c5, H5, W5, rois, sub, feat14, box7)
+            ops.roi_warp_split(c5f, self.c5, H5, W5, rois, sub, feat14, box7, img_hw=extents,
+                               level=C5_LEVEL)
 
     # ------------------------------------------------------------------ whole forward
-    def forward(self, data, im_info, keep_intermediate=False):
+    def forward(self, data, im_info, keep_intermediate=False, extents=None):
         """data fp32 (B,3,H,W) device, im_info fp32 (B,3) device [h, w, scale].
+        extents: None, or the int32 (B, 2) sizes of the images of a mixed-size batch, each in the
+        top-left corner of the zero-padded blob (normally im_info[:, :2]): every image then gets
+        the results it would get alone (device tensor: no host sync; host array: validated).
         Returns device tensors named after the blobs callers read (tools/demo.py:84-90):
         rois (B*300,5), mask_proposal (B*300,1,21,21), seg_cls_prob (B*300,21) and the `_ext`
         versions, plus roi_counts (B,) = number of real (non-padding) RoIs per image.
@@ -534,26 +610,28 @@ class MNCEngine:
         Precision mode 1 needs one exponent per tri-plane activation tensor: the first call
         measures them layer by layer on its own input (a few dozen host syncs, once) and freezes
         them; every later call is the sync-free launch sequence."""
+        extents = self._extents(data, extents)
         if not self._calibrated:
             self._calibrating = True
             try:
-                self._forward(data, im_info, False)
+                self._forward(data, im_info, False, extents)
             finally:
                 self._calibrating = False
             self._calibrated = True
-        return self._forward(data, im_info, keep_intermediate)
+        return self._forward(data, im_info, keep_intermediate, extents)
 
-    def _forward(self, data, im_info, keep_intermediate=False):
+    def _forward(self, data, im_info, keep_intermediate=False, extents=None):
         B = data.shape[0]
         out = {}
-        conv5_3, H5, W5, c5f, rois, roi_counts, res, rpn_out = self.rpn_rois(data, im_info, keep_intermediate)
+        conv5_3, H5, W5, c5f, rois, roi_counts, res, rpn_out = self.rpn_rois(data, im_info, keep_intermediate,
+                                                                             extents)
         c5 = self.c5
         R = B * ROIS_PER_IMAGE
         out["rois"] = rois
         out["roi_counts"] = roi_counts
         feat14 = self._act_buf("feat14", R, 14, 14, c5, exp_key="roi_feat")
         box7 = self._act_buf("box7", R, 7, 7, c5, exp_key="roi_feat")
-        self.roi_features(c5f, H5, W5, rois, 2, feat14, box7)
+        self.roi_features(c5f, H5, W5, rois, 2, feat14, box7, extents)
         s1 = self.head(feat14, box7, R, "s1")
         rois_ext = ops.stage_bridge(rois, s1["bbox_pred"], s1["seg_cls_prob"], im_info,
                                     ROIS_PER_IMAGE)
@@ -569,7 +647,7 @@ class MNCEngine:
             out["_mask_logits"] = s1["mask_logits"].clone()
             out["_mask_resize"] = s1["mask_resize"]
             out["_join"] = s1["join"].clone()
-        self.roi_features(c5f, H5, W5, rois_ext, 1, feat14, box7)
+        self.roi_features(c5f, H5, W5, rois_ext, 1, feat14, box7, extents)
         s2 = self.head(feat14, box7, R, "s2")
         for k in ("mask_proposal", "seg_cls_prob", "cls_prob", "bbox_pred"):
             out[k + "_ext"] = s2[k]
@@ -578,38 +656,42 @@ class MNCEngine:
             out["_mask_logits_ext"] = s2["mask_logits"].clone()
         return out
 
-    def detect(self, data, im_info, im_hw, im_scale):
+    def detect(self, data, im_info, im_hw, im_scale, extents=None):
         """forward + im_detect tail (tools/demo.py:92-100): boxes (B,600,4), masks (B,600,1,21,21),
-        scores (B,600,21), valid (B,600) uint8."""
-        o = self.forward(data, im_info)
+        scores (B,600,21), valid (B,600) uint8.  extents: see `forward`."""
+        o = self.forward(data, im_info, extents=extents)
         return self.detect_tail(o, data.shape[0], im_hw, im_scale) + (o,)
 
-    def detect_graphed(self, data, im_info, im_hw, im_scale, rec=None):
+    def detect_graphed(self, data, im_info, im_hw, im_scale, rec=None, extents=None):
         """`detect` replayed from a CUDA graph: the ~60 launches of a step (shapes, buffers and
         tensor maps are static once the exponents are calibrated) are captured on first use per
         (input buffers, shape) and re-issued with one cudaGraphLaunch -- what makes the single-image
         latency (BASELINE.json configs[0]) launch-bound no more.  Inputs are read from the tensors
         given at capture time: pass the same (persistent) tensors again, or others of the same
         shape, which are then copied in.  Returns the same views as `detect` (static buffers:
-        valid until the next call)."""
+        valid until the next call).  extents (see `forward`) are an input like im_info: one graph
+        serves every mix of image sizes that pads to the same blob shape."""
         if not hasattr(self, "_graphs"):
             self._graphs = {}
-        key = (tuple(data.shape), None if rec is None else rec.data_ptr())
+        extents = self._extents(data, extents)
+        ins = (data, im_info, im_hw, im_scale) + (() if extents is None else (extents,))
+        key = (tuple(data.shape), None if rec is None else rec.data_ptr(), extents is not None)
         ent = self._graphs.get(key)
         if ent is None:
-            st = [t if i == 0 else t.clone() for i, t in enumerate((data, im_info, im_hw, im_scale))]
+            st = [t if i == 0 else t.clone() for i, t in enumerate(ins)]
+            ex = st[4] if extents is not None else None
             for _ in range(2):                       # calibrates, sizes every buffer, loads kernels
-                self.detect(st[0], st[1], st[2], st[3])
+                self.detect(st[0], st[1], st[2], st[3], extents=ex)
             torch.cuda.synchronize(self.device)
             g = torch.cuda.CUDAGraph()
             # thread_local: a NCCL watchdog thread may poll events while this thread captures
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                o = self.forward(st[0], st[1])
+                o = self.forward(st[0], st[1], extents=ex)
                 outs = self.detect_tail(o, data.shape[0], st[2], st[3], rec=rec) + (o,)
             ent = (g, st, outs, self.last_record)
             self._graphs[key] = ent
         g, st, outs, last = ent
-        for dst, src in zip(st, (data, im_info, im_hw, im_scale)):
+        for dst, src in zip(st, ins):
             if dst.data_ptr() != src.data_ptr():
                 dst.copy_(src, non_blocking=True)
         g.replay()
@@ -633,6 +715,7 @@ class MNCEngine:
                 rec.zero_()          # the padding after counts[B] is never written by the kernel
         valid = self._buf.get("valid")
         if valid is None or valid.numel() < B * 2 * n:
+            self._drop_graphs(valid)
             valid = torch.empty(B * 2 * n, dtype=torch.uint8, device=self.device)
             self._buf["valid"] = valid
         valid = valid[:B * 2 * n].view(B, 2 * n)

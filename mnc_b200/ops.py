@@ -8,6 +8,7 @@ import ctypes
 import torch
 
 from ._lib import lib, ptr, cur_stream, check, c_int, c_ll, c_float
+from .dense import img_hw_arg
 
 c_double = ctypes.c_double
 lib.mnc_nms_workspace_bytes.restype = ctypes.c_longlong
@@ -69,8 +70,9 @@ def nms_sorted(boxes, counts, thresh, max_keep):
     key = (dev, nbytes)
     ws = _nms_ws.get(key)
     if ws is None:
+        # one workspace per size, kept: a captured CUDA graph (MNCEngine.detect_graphed) holds the
+        # address of the workspace it was captured with and replays into it
         ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        _nms_ws.clear()
         _nms_ws[key] = ws
     mk = max_keep if max_keep > 0 else n_max
     keep = _i32(problems, mk, device=dev)
@@ -103,9 +105,11 @@ def generate_anchors():
 
 
 def rpn_decode(cls, bbox, im_info, batch, H, W, layout, apply_softmax, feat_stride=16,
-               min_size=16.0):
+               min_size=16.0, img_hw=None, level=4):
     """layout 'nchw': cls (B,18,H,W), bbox (B,36,H,W); 'nhwc': one buffer (B,H,W,Cpad) where
-    channels [0,18) are cls and [18,54) bbox (then `bbox` is ignored)."""
+    channels [0,18) are cls and [18,54) bbox (then `bbox` is ignored).  img_hw: image sizes of a
+    mixed-size batch (device int32 (B, 2), input resolution; the map is `level` pools below it):
+    anchors outside their image are invalid."""
     dev = cls.device
     total = H * W * 9
     proposals = torch.empty((batch, total, 4), dtype=torch.float32, device=dev)
@@ -120,11 +124,14 @@ def rpn_decode(cls, bbox, im_info, batch, H, W, layout, apply_softmax, feat_stri
         ci, cc, cp = H * W * cpad, 1, cpad
         bi, bc, bp = ci, cc, cp
         bptr = ctypes.c_void_p(cls.data_ptr() + 18 * 4)
-    check(lib.mnc_rpn_decode(ptr(cls), c_ll(ci), c_ll(cc), c_ll(cp), bptr, c_ll(bi), c_ll(bc),
-                             c_ll(bp), ptr(im_info), c_int(batch), c_int(H), c_int(W),
-                             c_int(feat_stride), c_float(min_size), c_int(int(apply_softmax)),
-                             ptr(proposals), ptr(scores), ptr(valid), cur_stream()),
-          "mnc_rpn_decode")
+    args = (ptr(cls), c_ll(ci), c_ll(cc), c_ll(cp), bptr, c_ll(bi), c_ll(bc), c_ll(bp), ptr(im_info),
+            c_int(batch), c_int(H), c_int(W), c_int(feat_stride), c_float(min_size),
+            c_int(int(apply_softmax)), ptr(proposals), ptr(scores), ptr(valid))
+    if img_hw is None:
+        check(lib.mnc_rpn_decode(*args, cur_stream()), "mnc_rpn_decode")
+    else:
+        check(lib.mnc_rpn_decode2(*args, ptr(img_hw_arg(img_hw, batch)), c_int(level), cur_stream()),
+              "mnc_rpn_decode2")
     return proposals, scores, valid
 
 
@@ -142,10 +149,11 @@ def write_rois(sorted_boxes, keep, num_keep, max_rois, batch_index_mode):
 
 def proposals_from_rpn(cls, bbox, im_info, batch, H, W, layout, apply_softmax, pre_nms_top_n=6000,
                        post_nms_top_n=300, nms_thresh=0.7, min_size=16.0, batch_index_mode=True,
-                       return_intermediate=False):
-    """Whole ProposalLayer.forward on device (lib/pylayer/proposal_layer.py:52-175)."""
+                       return_intermediate=False, img_hw=None, level=4):
+    """Whole ProposalLayer.forward on device (lib/pylayer/proposal_layer.py:52-175).  img_hw /
+    level: image sizes of a mixed-size batch (rpn_decode)."""
     proposals, scores, valid = rpn_decode(cls, bbox, im_info, batch, H, W, layout, apply_softmax,
-                                          min_size=min_size)
+                                          min_size=min_size, img_hw=img_hw, level=level)
     total = H * W * 9
     n_sorted = min(pre_nms_top_n, total) if pre_nms_top_n > 0 else total
     if 8 * (1 << max(n_sorted - 1, 1).bit_length()) + 4 * total <= 200 * 1024:
@@ -263,25 +271,34 @@ def mask_pool_nchw(feat, mask, out=None):
     return out
 
 
-def roi_warp_split(feat, C, H, W, rois, sub, out14, out7, spatial_scale=0.0625):
-    """feat fp32 NHWC [B,H,W,C]; rois [R,5]; out14 split [2,R,14,14,C]; out7 split [2,R,7,7,C]."""
+def roi_warp_split(feat, C, H, W, rois, sub, out14, out7, spatial_scale=0.0625, img_hw=None, level=4):
+    """feat fp32 NHWC [B,H,W,C]; rois [R,5]; out14 split [2,R,14,14,C]; out7 split [2,R,7,7,C].
+    img_hw / level: image sizes of a mixed-size batch; samples are bounded by the RoI's image."""
     R = rois.shape[0]
     assert feat.dtype == torch.float32
-    check(lib.mnc_roi_warp_split(ptr(feat), c_int(C), c_int(H), c_int(W),
-                                 ptr(rois), c_int(R), c_int(sub), c_float(spatial_scale),
-                                 ptr(out14[0]), ptr(out14[1]), ptr(out7[0]), ptr(out7[1]),
-                                 cur_stream()), "mnc_roi_warp_split")
+    args = (ptr(feat), c_int(C), c_int(H), c_int(W), ptr(rois), c_int(R), c_int(sub),
+            c_float(spatial_scale), ptr(out14[0]), ptr(out14[1]), ptr(out7[0]), ptr(out7[1]))
+    if img_hw is None:
+        check(lib.mnc_roi_warp_split(*args, cur_stream()), "mnc_roi_warp_split")
+    else:
+        check(lib.mnc_roi_warp_split2(*args, ptr(img_hw_arg(img_hw, feat.shape[0])), c_int(level),
+                                      cur_stream()), "mnc_roi_warp_split2")
 
 
-def roi_warp_tri(feat, C, H, W, rois, sub, out14, out7, exp, spatial_scale=0.0625):
+def roi_warp_tri(feat, C, H, W, rois, sub, out14, out7, exp, spatial_scale=0.0625, img_hw=None,
+                 level=4):
     """roi_warp_split with tri-plane outputs (mnc_b200.dense.Tri) written with exponent `exp`."""
     R = rois.shape[0]
     assert feat.dtype == torch.float32
     out14.exp = out7.exp = int(exp)
-    check(lib.mnc_roi_warp_tri(ptr(feat), c_int(C), c_int(H), c_int(W), ptr(rois), c_int(R), c_int(sub),
-                               c_float(spatial_scale), c_float(2.0 ** exp), ptr(out14.h), ptr(out14.l),
-                               ptr(out14.c), ptr(out7.h), ptr(out7.l), ptr(out7.c), cur_stream()),
-          "mnc_roi_warp_tri")
+    args = (ptr(feat), c_int(C), c_int(H), c_int(W), ptr(rois), c_int(R), c_int(sub),
+            c_float(spatial_scale), c_float(2.0 ** exp), ptr(out14.h), ptr(out14.l), ptr(out14.c),
+            ptr(out7.h), ptr(out7.l), ptr(out7.c))
+    if img_hw is None:
+        check(lib.mnc_roi_warp_tri(*args, cur_stream()), "mnc_roi_warp_tri")
+    else:
+        check(lib.mnc_roi_warp_tri2(*args, ptr(img_hw_arg(img_hw, feat.shape[0])), c_int(level),
+                                    cur_stream()), "mnc_roi_warp_tri2")
 
 
 def mask_pool_tri(feat14, mask14, R, C, out7):
@@ -441,6 +458,35 @@ def prep_images(images_u8, scale, out=None, pixel_means=PIXEL_MEANS):
                               ctypes.c_double(scale), c_int(out_h), c_int(out_w), ptr(out),
                               cur_stream()), "mnc_prep_images")
     return out
+
+
+def blob_size_for(shape, scale):
+    """(rows, cols) of an image of `shape` (H, W, ...) in the blob at `scale` (cv2's rounding)."""
+    import numpy as np
+    return int(np.rint(shape[0] * scale)), int(np.rint(shape[1] * scale))
+
+
+def prep_images_ragged(packed_u8, offsets, src_hw, scales, out_h, out_w, out=None,
+                       pixel_means=PIXEL_MEANS):
+    """Images of different sizes in one launch (`im_list_to_blob` of `prep_im_for_blob` outputs):
+    packed_u8 a uint8 CUDA tensor holding image b (BGR HWC, src_hw[b]) at byte offsets[b]; image b
+    is prepared with scales[b] into the top-left corner of a zero-padded fp32 (B,3,out_h,out_w)
+    blob.  offsets / src_hw / scales: host sequences.  -> (blob, dst_hw int32 numpy (B, 2))."""
+    import numpy as np
+    B = len(scales)
+    dst = np.array([blob_size_for(hw, s) for hw, s in zip(src_hw, scales)], dtype=np.int32).reshape(B, 2)
+    if out is None:
+        out = torch.empty((B, 3, out_h, out_w), dtype=torch.float32, device=packed_u8.device)
+    off = np.ascontiguousarray(offsets, dtype=np.int64)
+    shw = np.ascontiguousarray(src_hw, dtype=np.int32).reshape(B, 2)
+    sc = np.ascontiguousarray(scales, dtype=np.float64)
+    if (shw.astype(np.int64).prod(axis=1) * 3 + off > packed_u8.numel()).any():
+        raise ValueError("prep_images_ragged: an image lies outside the packed buffer")
+    means = (ctypes.c_double * 3)(*pixel_means)
+    check(lib.mnc_prep_images_ragged(ptr(packed_u8), c_int(B), ptr(off), ptr(shw), ptr(sc), ptr(dst),
+                                     means, c_int(out_h), c_int(out_w), ptr(out), cur_stream()),
+          "mnc_prep_images_ragged")
+    return out, dst
 
 
 # ----------------------------------------------------------------------------- result rendering

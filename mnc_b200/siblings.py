@@ -22,8 +22,10 @@ from .engine import MNCEngine, ROIS_PER_IMAGE, NUM_CLASSES, MASK_SIZE
 class FasterRCNNEngine(MNCEngine):
     DEFAULT_PRECISION = "bf16x3"   # RoI producers of this graph write split-bf16 features
 
-    def forward(self, data, im_info, keep_intermediate=False):
+    def forward(self, data, im_info, keep_intermediate=False, extents=None):
         """-> rois (B*300,5), roi_counts (B,), cls_prob (B*300,21), bbox_pred (B*300,84)."""
+        if extents is not None:
+            raise NotImplementedError("mixed-size batches: the 5-stage MNCEngine only")
         B = data.shape[0]
         conv5_3, H5, W5, c5f, rois, roi_counts, res, _ = self.rpn_rois(data, im_info, keep_intermediate)
         c5, fc = self.c5, self.fc
@@ -45,9 +47,11 @@ class FasterRCNNEngine(MNCEngine):
             out["_proposal"] = res[2]
         return out
 
-    def detect(self, data, im_info, im_hw, im_scale):
+    def detect(self, data, im_info, im_hw, im_scale, extents=None):
         """forward + `_detection_forward` tail (TesterWrapper.py:226-237): per RoI 21 class scores
         and 21 decoded, clipped boxes.  -> scores (B,300,21), pred_boxes (B,300,84), valid."""
+        if extents is not None:
+            raise NotImplementedError("mixed-size batches: the 5-stage MNCEngine only")
         B = data.shape[0]
         o = self.forward(data, im_info)
         n = ROIS_PER_IMAGE
@@ -60,10 +64,12 @@ class FasterRCNNEngine(MNCEngine):
 class CFMEngine(MNCEngine):
     DEFAULT_PRECISION = "bf16x3"
 
-    def forward(self, data, rois, masks, keep_intermediate=False):
+    def forward(self, data, rois, masks, keep_intermediate=False, extents=None):
         """data fp32 (S,3,H,W) image pyramid; rois fp32 (R,5) [level,x1,y1,x2,y2] in the level's
         scaled coordinates; masks fp32 (R,1,14,14).  -> mask_prob (R,1,21,21), seg_cls_prob,
         cls_prob (R,21), bbox_pred (R,84)."""
+        if extents is not None:
+            raise NotImplementedError("mixed-size batches: the 5-stage MNCEngine only")
         S = data.shape[0]
         R = rois.shape[0]
         conv5_3, H5, W5 = self.trunk(data)
