@@ -410,6 +410,24 @@ int mnc_paste_instances(const float* boxes, int box_dim, const float* masks, con
                         float thresh, int* inst_img, int* cls_img, unsigned char* bgr,
                         void* stream);
 
+/* The same rendering straight from the outputs of batched mask voting (mnc_vote_select +
+ * mnc_mv_device), for images of different sizes in one launch: get_vis_dict (tools/demo.py:103-120)
+ * then _convert_pred_to_image per image.  n_res [batch], res_score / res_class [batch][max_results],
+ * result_box int32 [batch][max_results][4], result_mask [batch][max_results][M][M]; of the first
+ * n_res[b] results of image b those with res_score >= vis_thresh are painted, in order, the k-th of
+ * them as instance k.  img_hw int32 [batch][2] = (H_b, W_b); image b occupies pixels
+ * [pix_off[b], pix_off[b] + H_b*W_b) of inst_img / cls_img (int32, either may be NULL) and of bgr
+ * (uint8, 3 bytes a pixel, optional), packed without padding.  max_h / max_w: the largest H_b / W_b
+ * (launch shape).  thresh: the mask binarisation threshold (cfg.BINARIZE_THRESH).  Equal, bit for
+ * bit, to selecting those results and calling mnc_paste_instances image by image.  All device
+ * pointers. */
+int mnc_paste_voted_ragged(const int* n_res, const float* res_score, const int* res_class,
+                           const int* result_box, const float* result_mask, int batch,
+                           int max_results, int mask_size, const int* img_hw,
+                           const long long* pix_off, int max_h, int max_w, float vis_thresh,
+                           float thresh, int* inst_img, int* cls_img, unsigned char* bgr,
+                           void* stream);
+
 /* cv2.resize(mask, (bw, bh)) >= thresh for n predictions at once, as the AP^r evaluator does per
  * prediction (lib/utils/voc_eval.py:249-251).  rboxes int32 [n][4] already rounded; out is one
  * packed uint8 buffer, prediction i occupying bw_i*bh_i bytes (row-major) at offsets[i];

@@ -6,6 +6,8 @@
 HOST memory -- boxes (B,600,4), masks (B,600,1,21,21), scores (B,600,21), valid (B,600).
 Host<->device copies go through pinned staging buffers on the engine's stream.
 `Detector.mask_voting` is the batched `gpu_mask_voting` (lib/transform/mask_transform.py:213-286).
+`Detector.im_segment` goes from raw images to voted instances (and, optionally, the demo's rendered
+label images) in one call, with one small result record coming back to the host.
 """
 import numpy as np
 import torch
@@ -207,35 +209,60 @@ class Detector:
         (MNCEngine.clone_state), so that batch k+1's kernels fill batch k's wave tails and its
         low-occupancy proposal phase.  A yielded result is valid until the next iteration (its
         pinned buffers are reused two batches later)."""
-        dev = self.device
-        if getattr(self, "_s_in", None) is None:
-            self._s_in = torch.cuda.Stream(device=dev)
-            self._s_out = torch.cuda.Stream(device=dev)
-            self._slots = [None, None]
-            self._s_comp = [torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)]
-            self._engines = [self.engine, None]
+        return self._pipeline(batches)
+
+    def im_segment(self, images, max_per_image=100, render=False, vis_thresh=0.5):
+        """Raw images in, voted instances out: `im_detect` + `gpu_mask_voting`
+        (lib/transform/mask_transform.py:213-286) for every image of a batch, everything resident
+        on the device until one small record (plus, with render, the label images) is copied back.
+        images: a uint8 BGR (B, H, W, 3) array or tensor (as `im_detect_images` takes), or a list of
+        differently sized uint8 BGR (H_i, W_i, 3) images (as `im_detect_mixed` takes).  Returns a
+        list of B dicts, in input order: boxes int32 (k, 4), scores fp32 (k,), classes int32 (k,),
+        masks fp32 (k, 21, 21) -- every voted result, class-major as the reference's loops emit them
+        -- and the image's scale.  With render=True also the demo's images at the image's own size
+        (`_convert_pred_to_image` of `get_vis_dict(..., vis_thresh)`, tools/demo.py:153-164):
+        inst, cls int32 (H_i, W_i) and bgr uint8 (H_i, W_i, 3); vis_thresh affects these only."""
+        res, = self.im_segment_stream([images], max_per_image, render, vis_thresh)
+        return res
+
+    def im_segment_stream(self, batches, max_per_image=100, render=False, vis_thresh=0.5):
+        """Pipelined `im_segment`, built as `im_detect_stream` (two batches in flight, each slot
+        with its own engine state; frames in and results out on copy streams): an iterable of
+        batches of either form -> a generator of `im_segment` results per batch, in order."""
+        seg = dict(max_per_image=int(max_per_image), render=bool(render), vis_thresh=float(vis_thresh))
+        return self._pipeline(batches, seg)
+
+    def _pipeline(self, batches, seg=None):
+        """Two batches in flight (im_detect_stream); seg: the options of im_segment_stream, or None
+        for detect results."""
         pending = None
         for k, images_u8 in enumerate(batches):
-            cur = self._submit(k & 1, images_u8)
+            cur = self._submit(k & 1, images_u8, seg)
             if pending is not None:
                 yield self._collect(pending)
             pending = cur
         if pending is not None:
             yield self._collect(pending)
 
-    def _submit(self, slot, images_u8):
+    def _submit(self, slot, images_u8, seg=None):
         if isinstance(images_u8, (list, tuple)):
-            return self._submit_mixed(slot, images_u8)
+            return self._submit_mixed(slot, images_u8, seg)
         dev = self.device
         pinned_src = None
         if isinstance(images_u8, torch.Tensor):
-            assert images_u8.dtype == torch.uint8 and images_u8.is_contiguous()
+            if images_u8.dtype != torch.uint8 or not images_u8.is_contiguous():
+                raise ValueError("an image batch tensor must be contiguous uint8, got %s" % images_u8.dtype)
             if images_u8.is_pinned():
                 pinned_src = images_u8
             images_u8 = images_u8.numpy()
         images_u8 = np.ascontiguousarray(images_u8)
+        if images_u8.dtype != np.uint8 or images_u8.ndim != 4 or images_u8.shape[3] != 3 or \
+                min(images_u8.shape[1:3]) < 1:
+            raise ValueError("an image batch must be uint8 BGR (B, H, W, 3), got %s %s"
+                             % (images_u8.dtype, images_u8.shape))
         B, H, W, _ = images_u8.shape
-        assert B <= self.max_batch
+        if not 1 <= B <= self.max_batch:
+            raise ValueError("%d images in one batch, at most %d" % (B, self.max_batch))
         scale = ops.im_scale_for((H, W))
         out_h, out_w = int(np.rint(H * scale)), int(np.rint(W * scale))
         self._fit_input(out_h, out_w)
@@ -251,11 +278,17 @@ class Detector:
         sc = torch.full((B,), scale, dtype=torch.float32)
         prep = lambda: ops.prep_images(st["d_u8"][:B], scale, out=st["d_in"][:B])
         return self._issue(slot, st, eng, B, lambda: st["d_u8"][:B].copy_(pinned_src, non_blocking=True),
-                           prep, info, hw, sc, None, scale, images_u8.nbytes)
+                           prep, info, hw, sc, None, scale, images_u8.nbytes, seg)
 
     def _slot(self, slot):
         """Slot `slot`'s staging buffers (input blob sized like _d_in) and engine."""
         dev = self.device
+        if getattr(self, "_s_in", None) is None:
+            self._s_in = torch.cuda.Stream(device=dev)
+            self._s_out = torch.cuda.Stream(device=dev)
+            self._slots = [None, None]
+            self._s_comp = [torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)]
+            self._engines = [self.engine, None]
         st = self._slots[slot]
         if st is None:
             n_rec = ops.record_layout(self.max_batch, ROIS_PER_IMAGE)[3]
@@ -273,7 +306,7 @@ class Detector:
             eng = self._engines[slot] = self.engine.clone_state()
         return st, eng
 
-    def _submit_mixed(self, slot, images):
+    def _submit_mixed(self, slot, images, seg=None):
         mb = self._mixed_batch(images)
         B = mb["B"]
         self._fit_input(mb["H"], mb["W"])
@@ -286,11 +319,13 @@ class Detector:
         h2d = lambda: st["d_pack"][:nb].copy_(st["h_pack"][:nb], non_blocking=True)
         prep = lambda: ops.prep_images_ragged(st["d_pack"], mb["offsets"], mb["src_hw"], mb["scales"],
                                               mb["H"], mb["W"], out=st["d_in"][:B])
-        return self._issue(slot, st, eng, B, h2d, prep, info, hw, sc, mb["ext"], mb["scales"].copy(), nb)
+        return self._issue(slot, st, eng, B, h2d, prep, info, hw, sc, mb["ext"], mb["scales"].copy(), nb, seg)
 
-    def _issue(self, slot, st, eng, B, h2d, prep, info, hw, sc, ext, scale, in_bytes):
+    def _issue(self, slot, st, eng, B, h2d, prep, info, hw, sc, ext, scale, in_bytes, seg=None):
         """Queue one batch on slot `slot`: frames H2D on the copy stream (h2d), preparation (prep)
-        and the step on the slot's compute stream, the record D2H on the other copy stream."""
+        and the step on the slot's compute stream, the record D2H on the other copy stream.  With
+        seg (im_segment_stream), mask voting (and rendering) follow the step on the compute stream
+        and the voted record replaces the detect record on the way back."""
         dev = self.device
         with torch.cuda.device(dev), torch.cuda.stream(self._s_comp[slot]):
             main = torch.cuda.current_stream()                      # this slot's compute stream
@@ -310,30 +345,84 @@ class Detector:
             args = (st["d_in"][:B], info.to(dev, non_blocking=True), hw.to(dev, non_blocking=True),
                     sc.to(dev, non_blocking=True), None if ext is None else ext.to(dev, non_blocking=True))
             eng._amax_all.zero_()                                   # maxima of this step only
-            self._step(slot, args, B)
+            outs = self._step(slot, args, B)
+            job = None
+            if seg is not None:
+                job = self._seg_job(st, B, hw, scale, seg)
+                self._vote(st, outs, job, st["d_vrec"])
             ev_done = torch.cuda.Event()
             ev_done.record(main)
             with torch.cuda.stream(self._s_out):                    # record of this batch: D2H
                 self._s_out.wait_event(ev_done)
-                st["h_rec"][:n].copy_(st["d_rec"][:n], non_blocking=True)
+                if job is None:
+                    st["h_rec"][:n].copy_(st["d_rec"][:n], non_blocking=True)
+                else:
+                    n = job["n_rec"]
+                    st["h_vrec"][:n].copy_(st["d_vrec"][:n], non_blocking=True)
+                    if seg["render"]:
+                        nr = job["n_render"]
+                        st["h_rbuf"][:nr].copy_(st["d_rbuf"][:nr], non_blocking=True)
                 st["h_amax"].copy_(eng._amax_all, non_blocking=True)
                 st["out_done"] = torch.cuda.Event()
                 st["out_done"].record(self._s_out)
         self.h2d_bytes = in_bytes + (info.numel() + hw.numel() + sc.numel()) * 4
-        self.d2h_bytes = n * 4
+        if job is None:
+            self.d2h_bytes = n * 4
+        else:
+            self.d2h_bytes = job["n_rec"] * 4 + st["h_amax"].numel() * 4 + job["n_render"]
         # the exponents this step ran with (a captured graph keeps those of its capture)
-        return (slot, B, n, scale, args, dict(eng.exp))
+        return (slot, B, n, scale, args, dict(eng.exp), outs, job)
+
+    def _seg_job(self, st, B, hw, scale, seg):
+        """Device inputs and slot buffers (grown on demand) of the voting / rendering of one batch.
+        hw: host fp32 (B, 2) original image sizes."""
+        dev = self.device
+        hw_i = hw.to(torch.int32)
+        R = ops.default_vote_cap(seg["max_per_image"])
+        n_rec = ops.vote_record_layout(B, R, MASK_SIZE)[-1]
+        if st.get("d_vrec") is None or st["d_vrec"].numel() < n_rec:
+            st["d_vrec"] = torch.empty(n_rec, dtype=torch.int32, device=dev)
+            st["h_vrec"] = torch.empty(n_rec, dtype=torch.int32).pin_memory()
+        pix = hw_i[:, 0].long() * hw_i[:, 1].long()
+        pix_off = torch.cumsum(pix, 0) - pix
+        P = int(pix.sum())
+        job = dict(B=B, R=R, n_rec=n_rec, seg=seg, hw=hw_i.numpy(), pix_off=pix_off.numpy(), P=P,
+                   n_render=11 * P if seg["render"] else 0, scale=scale,
+                   d_hw=hw_i.to(dev, non_blocking=True))
+        if seg["render"]:
+            # one byte buffer, one copy back: inst int32[P] | cls int32[P] | bgr uint8[P][3]
+            if st.get("d_rbuf") is None or st["d_rbuf"].numel() < 11 * P:
+                st["d_rbuf"] = torch.empty(11 * P, dtype=torch.uint8, device=dev)
+                st["h_rbuf"] = torch.empty(11 * P, dtype=torch.uint8).pin_memory()
+            job["d_off"] = pix_off.to(dev, non_blocking=True)
+            job["max_hw"] = (int(job["hw"][:, 0].max()), int(job["hw"][:, 1].max()))
+        return job
+
+    def _vote(self, st, outs, job, d_vrec, R=None):
+        """Mask voting on the step outputs `outs` into the record d_vrec (R result slots per image,
+        default the job's), then, if asked for, rendering into the slot's render buffer."""
+        B, seg = job["B"], job["seg"]
+        R = job["R"] if R is None else R
+        boxes, masks, scores, valid = outs
+        views = ops.vote_record_views(d_vrec, B, R, MASK_SIZE)
+        ops.mask_voting(boxes, masks, scores, job["d_hw"], max_per_image=seg["max_per_image"],
+                        max_results=R, box_valid=valid, out=views)
+        if seg["render"]:
+            P, rb = job["P"], st["d_rbuf"]
+            ops.paste_voted_ragged(views, job["d_hw"], job["d_off"], job["max_hw"],
+                                   rb[:4 * P].view(torch.int32), rb[4 * P:8 * P].view(torch.int32),
+                                   rb[8 * P:11 * P], vis_thresh=seg["vis_thresh"])
 
     def _step(self, slot, args, B):
+        """One step of slot `slot` into its record -> (boxes, masks, scores, valid) device views."""
         eng, st = self._engines[slot], self._slots[slot]
         if self.use_graph:
-            eng.detect_graphed(*args[:4], rec=st["d_rec"], extents=args[4])
-        else:
-            o = eng.forward(args[0], args[1], extents=args[4])
-            eng.detect_tail(o, B, args[2], args[3], rec=st["d_rec"])
+            return eng.detect_graphed(*args[:4], rec=st["d_rec"], extents=args[4])[:4]
+        o = eng.forward(args[0], args[1], extents=args[4])
+        return eng.detect_tail(o, B, args[2], args[3], rec=st["d_rec"])
 
     def _collect(self, handle):
-        slot, B, n, scale, args, exp_used = handle
+        slot, B, n, scale, args, exp_used, outs, job = handle
         st, eng = self._slots[slot], self._engines[slot]
         st["out_done"].synchronize()
         # exponents re-measured since this batch was issued (on the other slot's batch): recompute
@@ -351,10 +440,16 @@ class Detector:
                         e._graphs.clear()
             with torch.cuda.device(dev), torch.cuda.stream(self._s_comp[slot]):
                 eng._amax_all.zero_()
-                self._step(slot, args, B)
-                st["h_rec"][:n].copy_(st["d_rec"][:n])
+                outs = self._step(slot, args, B)
+                if job is None:
+                    st["h_rec"][:n].copy_(st["d_rec"][:n])
+                else:
+                    self._vote(st, outs, job, st["d_vrec"])
+                    self._seg_to_host(st, job)
             torch.cuda.synchronize(dev)
             ok = eng.range_ok()
+        if job is not None:
+            return self._seg_results(slot, outs, job)
         counts, boxes, scores, masks = ops.record_views(st["h_rec"][:n], B, ROIS_PER_IMAGE)
         # valid flags from the counts (2 x RoIs per image: stage-1 rows, then stage-2 rows)
         per_stage = (counts.numpy() / 2).astype(np.int64)
@@ -362,8 +457,82 @@ class Detector:
         valid = (idx[None, :] < per_stage[:, None]).astype(np.uint8)
         return boxes.numpy(), masks.numpy(), scores.numpy(), valid, scale
 
+    @staticmethod
+    def _seg_to_host(st, job, d_vrec=None, h_vrec=None):
+        n = job["n_rec"] if d_vrec is None else d_vrec.numel()
+        (st["h_vrec"] if h_vrec is None else h_vrec)[:n].copy_((st["d_vrec"] if d_vrec is None else d_vrec)[:n])
+        if job["n_render"]:
+            st["h_rbuf"][:job["n_render"]].copy_(st["d_rbuf"][:job["n_render"]])
+
+    def _seg_results(self, slot, outs, job):
+        """The host side of a voted batch: results that did not fit the record's R slots per image
+        are voted again with twice the room (ops.mask_voting_checked's rule), then the per-image
+        results are cut out of the record (and the render buffer)."""
+        st, B, R, seg = self._slots[slot], job["B"], job["R"], job["seg"]
+        h_vrec = st["h_vrec"]
+        views = ops.vote_record_views(h_vrec, B, R, MASK_SIZE)
+        limit = outs[0].shape[1] * (NUM_CLASSES - 1)
+        while int(views["overflow"][0]) != 0:
+            if R >= limit:
+                raise ops.VotingOverflow("mask voting overflow at max_results = %d" % R)
+            R = min(2 * R, limit)
+            n = ops.vote_record_layout(B, R, MASK_SIZE)[-1]
+            d_vrec = torch.empty(n, dtype=torch.int32, device=self.device)
+            h_vrec = torch.empty(n, dtype=torch.int32)
+            with torch.cuda.device(self.device), torch.cuda.stream(self._s_comp[slot]):
+                # the step outputs stay valid until this slot's next submit
+                self._vote(st, outs, job, d_vrec, R)
+                self._seg_to_host(st, job, d_vrec, h_vrec)
+            self.d2h_bytes += n * 4 + job["n_render"]
+            views = ops.vote_record_views(h_vrec, B, R, MASK_SIZE)
+        n_res = views["n_res"].numpy()
+        cls, score = views["res_class"].numpy(), views["res_score"].numpy()
+        box, mask = views["result_box"].numpy(), views["result_mask"].numpy()
+        if seg["render"]:
+            P, rb = job["P"], st["h_rbuf"]
+            inst, clsi, bgr = (rb[:4 * P].view(torch.int32).numpy(), rb[4 * P:8 * P].view(torch.int32).numpy(),
+                               rb[8 * P:11 * P].numpy())
+        scale = job["scale"]
+        out = []
+        for b in range(B):
+            k = int(n_res[b])
+            r = dict(boxes=box[b, :k].copy(), scores=score[b, :k].copy(), classes=cls[b, :k].copy(),
+                     masks=mask[b, :k, 0].copy(),
+                     scale=float(scale if np.ndim(scale) == 0 else scale[b]))
+            if seg["render"]:
+                (H, W), o = job["hw"][b], int(job["pix_off"][b])
+                r["inst"] = inst[o:o + H * W].reshape(H, W).copy()
+                r["cls"] = clsi[o:o + H * W].reshape(H, W).copy()
+                r["bgr"] = bgr[3 * o:3 * (o + H * W)].reshape(H, W, 3).copy()
+            out.append(r)
+        return out
+
     def mask_voting(self, boxes, masks, scores, valid, im_hw, max_per_image=100):
         """Device-resident batched gpu_mask_voting on `engine.detect` outputs (device tensors)."""
         hw = torch.as_tensor(np.asarray(im_hw, dtype=np.int32)).to(self.device)
         return ops.mask_voting_checked(boxes, masks, scores, hw, max_per_image=max_per_image,
                                        box_valid=valid)
+
+
+def unpack_voting(result, num_classes=NUM_CLASSES):
+    """Voted results -> the reference's per-class format of `gpu_mask_voting`
+    (mask_transform.py:270-286): (list_result_mask, list_result_box), each a list over the
+    num_classes-1 foreground classes of (k,1,M,M) fp32 masks / (k,5) fp32 [box, score].
+    result: one image's result of `Detector.im_segment`; or the dict of device tensors that
+    `ops.mask_voting` returns for a batch, which gives a list of such pairs, one per image."""
+    if "n_res" in result:
+        n_res = result["n_res"].cpu().numpy()
+        cls, score = result["res_class"].cpu().numpy(), result["res_score"].cpu().numpy()
+        box, mask = result["result_box"].cpu().numpy(), result["result_mask"].cpu().numpy()
+        return [unpack_voting(dict(boxes=box[b, :k], scores=score[b, :k], classes=cls[b, :k],
+                                   masks=mask[b, :k]), num_classes)
+                for b, k in enumerate(n_res.astype(np.int64))]
+    masks = np.asarray(result["masks"])
+    M = masks.shape[-1]
+    boxes, scores, cls = np.asarray(result["boxes"]), np.asarray(result["scores"]), np.asarray(result["classes"])
+    list_mask, list_box = [], []
+    for c in range(1, num_classes):
+        sel = np.where(cls == c)[0]
+        list_mask.append(masks[sel].reshape(-1, 1, M, M).astype(np.float32))
+        list_box.append(np.hstack((boxes[sel].astype(np.float32), scores[sel, None].astype(np.float32))))
+    return list_mask, list_box

@@ -21,7 +21,12 @@ namespace mnc {
 struct InstRec {
   int x1, y1, x2, y2;  // np.round(box).astype(int), clipped to the image (vis_seg.py:106-114)
   int cls;
+  int id;              // position among the painted entries of its chunk, 1-based (0: not painted)
 };
+
+__device__ __forceinline__ int box_coord(float v) { return static_cast<int>(rintf(v)); }
+// voted boxes are integers already (mnc_mv_device); rintf of their fp32 copy is the same value
+__device__ __forceinline__ int box_coord(int v) { return v; }
 
 __device__ __forceinline__ void cv_tap(int d, double scale, int n, int& i0, int& i1, float& a0,
                                        float& a1) {
@@ -49,37 +54,81 @@ __device__ __forceinline__ bool in_edge_band(int v, int a) { return a >= 1 && (v
 
 constexpr int kRenderChunk = 256;
 
-// grid (ceil(W/128), H, batch); 128 threads, one pixel each.
+// grid (ceil(max W/128), max H, batch); 128 threads, one pixel each.
+// img_hw == nullptr: every image is H x W and image b starts at pixel b*H*W.  Otherwise image b is
+// img_hw[b] = (H_b, W_b) starting at pixel pix_off[b] (images packed without padding); blocks
+// outside their image return at once.
+// scores == nullptr: the counts[b] entries are all painted, entry i as instance i+1.  Otherwise
+// only the entries with scores[i] >= vis_thresh are, in order, numbered 1, 2, ... by their position
+// among them (get_vis_dict, tools/demo.py:103-120, then _convert_pred_to_image).
+template <typename BoxT>
 __global__ void __launch_bounds__(128)
-paste_instances_kernel(const float* __restrict__ boxes, int box_dim, const float* __restrict__ masks,
-                       const int* __restrict__ cls, const int* __restrict__ counts, int max_n, int M,
-                       int H, int W, float thresh, int* __restrict__ inst_img,
-                       int* __restrict__ cls_img, unsigned char* __restrict__ bgr) {
+paste_instances_kernel(const BoxT* __restrict__ boxes, int box_dim, const float* __restrict__ masks,
+                       const int* __restrict__ cls, const int* __restrict__ counts,
+                       const float* __restrict__ scores, float vis_thresh, int max_n, int M,
+                       const int* __restrict__ img_hw, const long long* __restrict__ pix_off, int H,
+                       int W, float thresh, int* __restrict__ inst_img, int* __restrict__ cls_img,
+                       unsigned char* __restrict__ bgr) {
   __shared__ InstRec recs[kRenderChunk];
+  __shared__ int s_warp[4];
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
   const int y = blockIdx.y;
   const int b = blockIdx.z;
+  long long img_off = static_cast<long long>(b) * H * W;
+  if (img_hw) {
+    H = img_hw[2 * b];
+    W = img_hw[2 * b + 1];
+    img_off = pix_off[b];
+    if (y >= H || static_cast<int>(blockIdx.x * blockDim.x) >= W) return;   // block-uniform
+  }
   const int n = min(counts[b], max_n);
-  const float* pboxes = boxes + static_cast<long long>(b) * max_n * box_dim;
+  const BoxT* pboxes = boxes + static_cast<long long>(b) * max_n * box_dim;
   const float* pmasks = masks + static_cast<long long>(b) * max_n * M * M;
   const int* pcls = cls + static_cast<long long>(b) * max_n;
+  const float* pscores = scores ? scores + static_cast<long long>(b) * max_n : nullptr;
+  int kept_total = n;
+  if (pscores) {
+    kept_total = 0;
+    for (int base = 0; base < n; base += blockDim.x) {
+      const int i = base + threadIdx.x;
+      kept_total += __syncthreads_count(i < n && pscores[i] >= vis_thresh);
+    }
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 
   int inst_val = 0, cls_val = 0;
   bool inst_done = false, cls_done = false;
+  int kept_after = 0;   // painted entries in [hi, n)
   // chunks from the end of the list towards its start
   for (int hi = n; hi > 0; hi -= kRenderChunk) {
     const int lo = max(hi - kRenderChunk, 0);
     __syncthreads();
-    for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) {
-      const float* bx = pboxes + static_cast<long long>(i) * box_dim;
+    // two rounds of 128 entries (kRenderChunk = 2 * blockDim.x): every thread takes part in both
+    int kept_chunk = 0;
+    for (int i = lo + threadIdx.x; i < lo + kRenderChunk; i += blockDim.x) {
+      const bool in = i < hi;
+      const bool keep = in && (!pscores || pscores[i] >= vis_thresh);
+      const unsigned bal = __ballot_sync(0xffffffffu, keep);
+      if (lane == 0) s_warp[warp] = __popc(bal);
+      __syncthreads();
+      int id = kept_chunk + __popc(bal & ((2u << lane) - 1u));   // inclusive count in the chunk
+      for (int w = 0; w < warp; ++w) id += s_warp[w];
+      kept_chunk += s_warp[0] + s_warp[1] + s_warp[2] + s_warp[3];
+      __syncthreads();
+      if (!in) continue;
+      const BoxT* bx = pboxes + static_cast<long long>(i) * box_dim;
       InstRec r;
-      r.x1 = min(max(static_cast<int>(rintf(bx[0])), 0), W - 1);
-      r.y1 = min(max(static_cast<int>(rintf(bx[1])), 0), H - 1);
-      r.x2 = min(max(static_cast<int>(rintf(bx[2])), 0), W - 1);
-      r.y2 = min(max(static_cast<int>(rintf(bx[3])), 0), H - 1);
+      r.x1 = min(max(box_coord(bx[0]), 0), W - 1);
+      r.y1 = min(max(box_coord(bx[1]), 0), H - 1);
+      r.x2 = min(max(box_coord(bx[2]), 0), W - 1);
+      r.y2 = min(max(box_coord(bx[3]), 0), H - 1);
       r.cls = pcls[i];
+      r.id = id;
+      if (!keep) r.x2 = r.x1 - 1;   // filtered out: an empty box paints nothing
       recs[i - lo] = r;
     }
+    const int id_base = kept_total - kept_after - kept_chunk;   // painted entries before lo
+    kept_after += kept_chunk;
     __syncthreads();
     const bool all_done = (x >= W) || (inst_done && cls_done);
     if (__syncthreads_and(all_done)) break;
@@ -109,7 +158,7 @@ paste_instances_kernel(const float* __restrict__ boxes, int box_dim, const float
       const float v = __fadd_rn(__fmul_rn(r0, ay0), __fmul_rn(r1, ay1));
       if (v >= thresh) {
         if (!inst_done) {
-          inst_val = i + 1;
+          inst_val = id_base + r.id;
           inst_done = true;
         }
         if (!cls_done) {
@@ -120,7 +169,7 @@ paste_instances_kernel(const float* __restrict__ boxes, int box_dim, const float
     }
   }
   if (x >= W) return;
-  const long long o = (static_cast<long long>(b) * H + y) * W + x;
+  const long long o = img_off + static_cast<long long>(y) * W + x;
   if (inst_img) inst_img[o] = inst_val;
   if (cls_img) cls_img[o] = cls_val;
   if (bgr) {
@@ -175,8 +224,25 @@ extern "C" int mnc_paste_instances(const float* boxes, int box_dim, const float*
   if (batch <= 0 || max_n < 0 || box_dim < 4 || mask_size <= 0 || H <= 0 || W <= 0)
     return MNC_ERR_ARG;
   dim3 grid((W + 127) / 128, H, batch);
-  mnc::paste_instances_kernel<<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(
-      boxes, box_dim, masks, cls, counts, max_n, mask_size, H, W, thresh, inst_img, cls_img, bgr);
+  mnc::paste_instances_kernel<float><<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      boxes, box_dim, masks, cls, counts, nullptr, 0.f, max_n, mask_size, nullptr, nullptr, H, W,
+      thresh, inst_img, cls_img, bgr);
+  return cudaGetLastError() == cudaSuccess ? MNC_OK : MNC_ERR_CUDA;
+}
+
+extern "C" int mnc_paste_voted_ragged(const int* n_res, const float* res_score, const int* res_class,
+                                      const int* result_box, const float* result_mask, int batch,
+                                      int max_results, int mask_size, const int* img_hw,
+                                      const long long* pix_off, int max_h, int max_w,
+                                      float vis_thresh, float thresh, int* inst_img, int* cls_img,
+                                      unsigned char* bgr, void* stream) {
+  if (batch <= 0 || max_results < 0 || mask_size <= 0 || max_h <= 0 || max_w <= 0 || !n_res ||
+      !res_score || !img_hw || !pix_off)
+    return MNC_ERR_ARG;
+  dim3 grid((max_w + 127) / 128, max_h, batch);
+  mnc::paste_instances_kernel<int><<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      result_box, 4, result_mask, res_class, n_res, res_score, vis_thresh, max_results, mask_size,
+      img_hw, pix_off, max_h, max_w, thresh, inst_img, cls_img, bgr);
   return cudaGetLastError() == cudaSuccess ? MNC_OK : MNC_ERR_CUDA;
 }
 

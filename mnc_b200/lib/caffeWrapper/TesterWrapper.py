@@ -25,7 +25,7 @@ import numpy as np
 import torch
 
 from mnc_b200 import ops
-from mnc_b200.api import Detector
+from mnc_b200.api import Detector, unpack_voting
 from mnc_config import cfg
 from nms.nms_wrapper import apply_nms_mask_single
 
@@ -247,25 +247,11 @@ class TesterWrapper(object):
         return all_boxes, all_masks
 
     def _vote_batch(self, ims):
-        """forward + gpu_mask_voting for one batch of equally sized images, everything resident
-        on the device until the voted results come back.  -> per image (list_mask, list_box) in
-        the format `gpu_mask_voting` returns (mask_transform.py:270-286)."""
-        det = self.detector
-        B, H, W = ims.shape[:3]
-        dev = self.device
-        scale = ops.im_scale_for((H, W))
-        out_h, out_w = int(np.rint(H * scale)), int(np.rint(W * scale))
-        det._fit_input(out_h, out_w)
-        with torch.cuda.device(dev):
-            d_u8 = torch.from_numpy(ims).to(dev)
-            ops.prep_images(d_u8, scale, out=det._d_in[:B])
-            info = torch.tensor([[out_h, out_w, scale]] * B, dtype=torch.float32, device=dev)
-            hw = torch.tensor([[H, W]] * B, dtype=torch.float32, device=dev)
-            sc = torch.full((B,), scale, dtype=torch.float32, device=dev)
-            boxes, masks, scores, valid, _ = det.engine.detect_checked(det._d_in[:B], info, hw, sc)
-            vote = det.mask_voting(boxes, masks, scores, valid, [[H, W]] * B,
-                                   max_per_image=self.max_per_image)
-            return unpack_voting(vote, self.num_classes)
+        """forward + gpu_mask_voting for one batch of equally sized images (Detector.im_segment).
+        -> per image (list_mask, list_box) in the format `gpu_mask_voting` returns
+        (mask_transform.py:270-286)."""
+        res = self.detector.im_segment(ims, max_per_image=self.max_per_image)
+        return [unpack_voting(r, self.num_classes) for r in res]
 
 
 class _ClassBook(object):
@@ -289,25 +275,3 @@ class _ClassBook(object):
                 heapq.heappop(heap)
             self.thresh[j] = heap[0]
         return inds
-
-
-def unpack_voting(vote, num_classes):
-    """Device voting results -> per image (list_result_mask, list_result_box), each a list over
-    the num_classes-1 foreground classes of (k,1,M,M) fp32 masks / (k,5) fp32 [box, score]."""
-    n_res = vote["n_res"].cpu().numpy()
-    rcls = vote["res_class"].cpu().numpy()
-    rscore = vote["res_score"].cpu().numpy()
-    rmask = vote["result_mask"].cpu().numpy()
-    rbox = vote["result_box"].cpu().numpy()
-    out = []
-    M = rmask.shape[-1]
-    for b in range(len(n_res)):
-        k = int(n_res[b])
-        list_mask, list_box = [], []
-        for c in range(1, num_classes):
-            sel = np.where(rcls[b, :k] == c)[0]
-            list_mask.append(rmask[b, sel].reshape(-1, 1, M, M).astype(np.float32))
-            list_box.append(np.hstack((rbox[b, sel].astype(np.float32),
-                                       rscore[b, sel, None].astype(np.float32))))
-        out.append((list_mask, list_box))
-    return out

@@ -61,13 +61,14 @@ def gather_boxes(src, src_stride, src_outer_stride, inner, order, counts, n_out,
 _nms_ws = {}
 
 
-def nms_sorted(boxes, counts, thresh, max_keep):
+def nms_sorted(boxes, counts, thresh, max_keep, per_stream=False):
     """boxes fp32 [problems, n_max, 4] score-sorted; counts int32 [problems] or None.
-    -> (keep int32 [problems, max_keep], num int32 [problems])."""
+    per_stream: a workspace of its own for the current stream, for callers that run on several
+    streams at once.  -> (keep int32 [problems, max_keep], num int32 [problems])."""
     problems, n_max, stride = boxes.shape
     dev = boxes.device
     nbytes = lib.mnc_nms_workspace_bytes(c_int(n_max), c_int(problems))
-    key = (dev, nbytes)
+    key = (dev, nbytes) + ((torch.cuda.current_stream(dev).cuda_stream,) if per_stream else ())
     ws = _nms_ws.get(key)
     if ws is None:
         # one workspace per size, kept: a captured CUDA graph (MNCEngine.detect_graphed) holds the
@@ -214,6 +215,29 @@ def record_views(rec, B, n, msz=441, ncls=21):
             rec[om:end].view(B, 2 * n, 1, side, side))
 
 
+def vote_record_layout(B, R, M=21):
+    """Offsets (in 4-byte elements) of the sections of a mask-voting result record and its length:
+    n_res[B] | overflow | class[B][R] | score[B][R] | box[B][R][4] | mask[B][R][M*M].  Integer
+    sections hold int32 bit patterns; every section starts on a 16-byte boundary."""
+    up = lambda v: (v + 3) // 4 * 4
+    o_over = up(B)
+    o_class = up(o_over + 1)
+    o_score = o_class + up(B * R)
+    o_box = o_score + up(B * R)
+    o_mask = o_box + B * R * 4
+    return o_over, o_class, o_score, o_box, o_mask, o_mask + B * R * M * M
+
+
+def vote_record_views(rec, B, R, M=21):
+    """Views of a record of `vote_record_layout(B, R, M)` elements (4-byte dtype; device or host):
+    the keys of the dict `mask_voting` returns that the record holds, each in its dtype."""
+    oo, oc, os_, ob, om, end = vote_record_layout(B, R, M)
+    i32, f32 = rec[:end].view(torch.int32), rec[:end].view(torch.float32)
+    return dict(n_res=i32[:B], overflow=i32[oo:oo + 1], res_class=i32[oc:oc + B * R].view(B, R),
+                res_score=f32[os_:os_ + B * R].view(B, R), result_box=i32[ob:om].view(B, R, 4),
+                result_mask=f32[om:end].view(B, R, 1, M, M))
+
+
 def detect_tail(o, B, n, im_scale, im_hw, rec, valid):
     """im_detect tail into the record buffer `rec` (fp32, record_layout(B, n)[3] floats) and
     `valid` (uint8 [B, 2n]).  Returns (counts, boxes, scores, masks) views of rec."""
@@ -354,11 +378,18 @@ class VotingOverflow(RuntimeError):
     pass
 
 
+def default_vote_cap(max_per_image):
+    """Result slots per image a voting call starts with (more only after an overflow)."""
+    return max(128, max_per_image + 28)
+
+
 def mask_voting(boxes, masks, scores, im_hw, max_per_image=100, nms_thresh=0.3, iou_thresh=0.5,
-                max_results=128, box_valid=None):
+                max_results=128, box_valid=None, out=None):
     """Batched device pipeline of gpu_mask_voting (lib/transform/mask_transform.py:213-286).
     boxes [B,nb,4] fp32, masks [B,nb,1,M,M] fp32, scores [B,nb,ncls] fp32, im_hw [B,2] int32.
     box_valid: optional uint8 [B,nb]; rows with 0 are padding and take no part.
+    out: optional `vote_record_views(rec, B, max_results, M)`; the results are written there (one
+    record, one copy to the host) instead of into fresh tensors.
     Returns dict of device tensors: n_res [B], class_bar [B,ncls-1], res_score [B,max_results],
     res_class, result_mask [B,max_results,1,M,M], result_box [B,max_results,4] int32, plus the
     candidate lists."""
@@ -373,13 +404,24 @@ def mask_voting(boxes, masks, scores, im_hw, max_per_image=100, nms_thresh=0.3, 
     order, n_valid = rank_sort_desc(scores[:, :, 1:], nb, nprob, outer_stride=nb * ncls,
                                     inner_stride=1, inner=ncls - 1, key_stride=ncls, valid=valid_p)
     sorted_boxes, counts = gather_boxes(boxes, 4, nb * 4, ncls - 1, order, n_valid, nb, nprob)
-    keep, num = nms_sorted(sorted_boxes, counts, nms_thresh, min(max_per_image, nb))
+    # two pipelined batches vote at once on two streams (Detector.im_segment_stream)
+    keep, num = nms_sorted(sorted_boxes, counts, nms_thresh, min(max_per_image, nb), per_stream=True)
     res_idx = _i32(B, max_results, device=dev)
-    res_cls = _i32(B, max_results, device=dev)
-    res_score = torch.zeros((B, max_results), dtype=torch.float32, device=dev)
-    n_res = _i32(B, device=dev)
     class_bar = _i32(B, ncls - 1, device=dev)
-    overflow = torch.zeros(1, dtype=torch.int32, device=dev)
+    if out is None:
+        res_cls = _i32(B, max_results, device=dev)
+        res_score = torch.zeros((B, max_results), dtype=torch.float32, device=dev)
+        n_res = _i32(B, device=dev)
+        overflow = torch.zeros(1, dtype=torch.int32, device=dev)
+        out_mask = torch.zeros((B, max_results, 1, M, M), dtype=torch.float32, device=dev)
+        out_box = torch.zeros((B, max_results, 4), dtype=torch.int32, device=dev)
+    else:
+        if out["res_score"].shape != (B, max_results) or out["result_mask"].shape[-1] != M:
+            raise ValueError("mask_voting: out= views of another shape")
+        res_cls, res_score, n_res, overflow = out["res_class"], out["res_score"], out["n_res"], out["overflow"]
+        out_mask, out_box = out["result_mask"], out["result_box"]
+        for t in (res_score, overflow, out_mask, out_box):
+            t.zero_()
     check(lib.mnc_vote_select(ptr(scores), c_int(nb), c_int(ncls), ptr(order), ptr(keep),
                               c_int(keep.shape[1]), ptr(num), c_int(max_per_image),
                               c_int(max_results), c_int(B), ptr(res_idx), ptr(res_cls),
@@ -396,8 +438,6 @@ def mask_voting(boxes, masks, scores, im_hw, max_per_image=100, nms_thresh=0.3, 
                                   ptr(cand_begin), ptr(cand_end), cur_stream()),
           "mnc_vote_candidates")
     bbox_ws = _i32(B * max_results * 4 + B, device=dev)   # tight boxes + per-image range flag
-    out_mask = torch.zeros((B, max_results, 1, M, M), dtype=torch.float32, device=dev)
-    out_box = torch.zeros((B, max_results, 4), dtype=torch.int32, device=dev)
     check(lib.mnc_mv_device(ptr(boxes), ptr(masks), c_int(nb), c_int(4), c_int(M), ptr(cand_inds),
                             ptr(cand_w), c_ll(max_results * nb), ptr(cand_begin), ptr(cand_end),
                             ptr(n_res), c_int(max_results), c_int(B), ptr(im_hw), ptr(bbox_ws),
@@ -419,7 +459,7 @@ def mask_voting_checked(boxes, masks, scores, im_hw, max_per_image=100, box_vali
     """mask_voting that never truncates: the reference keeps EVERY kept row whose score ties the
     global threshold (mask_transform.py:258), so when more rows tie than `max_results` has slots
     the device reports it and the call is repeated with room (one host read of a 4-byte flag)."""
-    cap = kw.pop("max_results", max(128, max_per_image + 28))
+    cap = kw.pop("max_results", default_vote_cap(max_per_image))
     nb = boxes.shape[1]
     while True:
         r = mask_voting(boxes, masks, scores, im_hw, max_per_image=max_per_image, max_results=cap,
@@ -509,6 +549,24 @@ def paste_instances(boxes, masks, cls, counts, H, W, thresh=0.4, want_bgr=False)
                                   ptr(inst), ptr(clsi), ptr(bgr), cur_stream()),
           "mnc_paste_instances")
     return (inst, clsi, bgr) if want_bgr else (inst, clsi)
+
+
+def paste_voted_ragged(vote, img_hw, pix_off, max_hw, inst, cls, bgr, vis_thresh=0.5, thresh=0.4):
+    """`select_for_display` + `paste_instances` for images of different sizes in one launch,
+    straight from the outputs of `mask_voting` (its dict, or `vote_record_views` of its record).
+    img_hw: device int32 (B, 2) image sizes; pix_off: device int64 (B,) first pixel of each image
+    in the packed outputs; max_hw: host (max H, max W).  inst, cls int32 and bgr uint8 device
+    tensors of P, P and 3P elements, P = sum of H_b * W_b (inst / cls may be None): image b is
+    written to pixels [pix_off[b], pix_off[b] + H_b * W_b)."""
+    score = vote["res_score"]
+    B, R = score.shape
+    M = vote["result_mask"].shape[-1]
+    check(lib.mnc_paste_voted_ragged(ptr(vote["n_res"]), ptr(score), ptr(vote["res_class"]),
+                                     ptr(vote["result_box"]), ptr(vote["result_mask"]), c_int(B),
+                                     c_int(R), c_int(M), ptr(img_hw), ptr(pix_off),
+                                     c_int(int(max_hw[0])), c_int(int(max_hw[1])),
+                                     c_float(vis_thresh), c_float(thresh), ptr(inst), ptr(cls),
+                                     ptr(bgr), cur_stream()), "mnc_paste_voted_ragged")
 
 
 def select_for_display(vote, vis_thresh=0.5):

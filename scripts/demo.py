@@ -18,7 +18,6 @@ import cv2
 import numpy as np
 import torch
 
-from mnc_b200 import ops
 from mnc_b200.api import Detector
 
 
@@ -50,31 +49,17 @@ def main():
     by_shape = {}
     for p, im in frames:
         by_shape.setdefault(im.shape, []).append((p, im))
-    for shape, group in by_shape.items():
-        H, W = shape[:2]
+    for group in by_shape.values():
         for s in range(0, len(group), args.max_batch):
             chunk = group[s:s + args.max_batch]
-            ims = np.stack([im for _, im in chunk])
-            B = len(chunk)
-            scale = ops.im_scale_for((H, W))
-            out_h, out_w = int(np.rint(H * scale)), int(np.rint(W * scale))
-            det._fit_input(out_h, out_w)
-            d_u8 = torch.from_numpy(ims).to(dev)
-            ops.prep_images(d_u8, scale, out=det._d_in[:B])
-            info = torch.tensor([[out_h, out_w, scale]] * B, dtype=torch.float32, device=dev)
-            hw = torch.tensor([[H, W]] * B, dtype=torch.float32, device=dev)
-            sc = torch.full((B,), scale, dtype=torch.float32, device=dev)
-            boxes, masks, scores, valid, _ = det.engine.detect_checked(det._d_in[:B], info, hw, sc)
-            vote = det.mask_voting(boxes, masks, scores, valid, [[H, W]] * B, max_per_image=100)
-            vb, vm, vc, cnt = ops.select_for_display(vote, vis_thresh=args.vis_thresh)
-            inst, cls, bgr = ops.paste_instances(vb, vm, vc, cnt, H, W, want_bgr=True)
-            bgr = bgr.cpu().numpy()
-            for i, (path, im) in enumerate(chunk):
+            res = det.im_segment(np.stack([im for _, im in chunk]), render=True, vis_thresh=args.vis_thresh)
+            for (path, im), r in zip(chunk, res):
                 name = os.path.splitext(os.path.basename(path))[0]
-                cv2.imwrite(os.path.join(args.out, "cls_%s.png" % name), bgr[i])
-                blend = cv2.addWeighted(im, 0.2, bgr[i], 0.8, 0.0)
+                cv2.imwrite(os.path.join(args.out, "cls_%s.png" % name), r["bgr"])
+                blend = cv2.addWeighted(im, 0.2, r["bgr"], 0.8, 0.0)
                 cv2.imwrite(os.path.join(args.out, "final_%s.jpg" % name), blend)
-                print("%s: %d instances drawn (%d voted)" % (path, int(cnt[i]), int(vote["n_res"][i])))
+                drawn = int((r["scores"] >= args.vis_thresh).sum())
+                print("%s: %d instances drawn (%d voted)" % (path, drawn, len(r["scores"])))
 
 
 if __name__ == "__main__":
